@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Benchmark of the Siegel pair-distance hot path (BASELINE.json metric: pairs/s forward+backward).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--n 4] [--kind upper]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--n 4] [--kind upper] [--dump-outputs DIR]
 
 Workload (config.workload) = BASELINE.json configs[4], the distance microbench: a table of 2^20 random points
 and ONE BATCH OF 64M (2^26) random index pairs per step, manifold `--kind` with n x n matrices, forward +
@@ -13,6 +13,8 @@ step ends with the one collective of the path, the NCCL all-reduce (average) of 
 and graph distances copied from pinned host memory and the loss read back, inside the timed region.
 A second record, `n10`, repeats the measurement for upper / fmin / n = 10 (the other size BASELINE.json's metric
 names) on a smaller batch.
+`--dump-outputs DIR` writes what the last timed step of the headline record returned to its caller as float64 .npy
+files (see dump_outputs); the inputs depend only on the arguments, so two builds can be compared output for output.
 """
 import argparse
 import json
@@ -26,11 +28,15 @@ import time
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
 
+import numpy as np  # noqa: E402
 import torch  # noqa: E402
 
 GLOBAL_PAIRS = 1 << 26          # BASELINE.json configs[4]: 64M random pairs per batch
 CHUNK_PAIRS = 1 << 23           # pairs per API call (saved unit gradients of a chunk: 2.7 GB at n = 4)
 N10_GLOBAL_PAIRS = 1 << 23      # batch of the n = 10 side record (a step is ~0.1-0.2 s on one GPU)
+DUMP_SEED = 20261020            # --dump-outputs: seed of the sampled pairs and table rows
+DUMP_DIST_MAX = 1 << 20         # --dump-outputs: at most this many distances (8 MB)
+DUMP_GRAD_BYTES = 48 << 20      # --dump-outputs: at most this many bytes of table-gradient rows (64 MB in all)
 
 
 def chunk_pairs_for(n):
@@ -180,6 +186,31 @@ def reference_loss(graph_dist, manifold_dist):
     return torch.abs(torch.pow(manifold_dist / graph_dist, 2) - 1).sum()
 
 
+def _sample(count, keep):
+    """sorted positions of a fixed, seeded sample of `keep` out of `count` (all of them when they fit)"""
+    if count <= keep:
+        return torch.arange(count)
+    return torch.randperm(count, generator=torch.Generator().manual_seed(DUMP_SEED))[:keep].sort().values
+
+
+def dump_outputs(out_dir, dists, loss, table_grad):
+    """What one step of the timed path hands its caller, as float64 .npy files in out_dir:
+    loss.npy        (1,)            the step's distortion loss (sum over the chunks)
+    dist.npy        (m,)            manifold distances at a seeded sample of this rank's pair positions
+    table_grad.npy  (r, *row shape) table.grad at a seeded sample of the table rows (after the all-reduce)
+    The samples depend only on the batch and table sizes; together the files stay below 64 MB."""
+    os.makedirs(out_dir, exist_ok=True)
+    d = torch.cat([x.reshape(-1) for x in dists])
+    d = d[_sample(d.numel(), DUMP_DIST_MAX).to(d.device)]
+    rows = table_grad.shape[0]
+    row_bytes = table_grad[0].numel() * 8
+    g = table_grad[_sample(rows, max(1, DUMP_GRAD_BYTES // row_bytes)).to(table_grad.device)]
+    arrays = {"loss": loss.reshape(1), "dist": d, "table_grad": g}
+    for name, t in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), t.detach().to("cpu", torch.float64).numpy())
+    return sorted(arrays)
+
+
 def make_manifold(kind, n, metric, dev):
     from sympa_b200 import BoundedDomainManifold, MetricType, SymmetricPositiveDefinite, UpperHalfManifold
     if kind == "spd":
@@ -205,8 +236,9 @@ def our_launches_per_chunk(kind, n, rows, b, dev, world, single_chunk=True):
 
 
 def measure(kind, n, metric, rows, global_pairs, steps, warmup, rank, world, local, dev, per_kernel=True, fused=True,
-            e2e=True):
-    """pairs/s of one configuration: resident step, per-kernel times, fused step, end-to-end step."""
+            e2e=True, dump_dir=None):
+    """pairs/s of one configuration: resident step, per-kernel times, fused step, end-to-end step.  dump_dir: rank 0
+    writes the outputs of the last timed resident step there (dump_outputs)."""
     import torch.distributed as dist
     from sympa_b200 import _lib, ops
     from sympa_b200 import distributed as sd
@@ -244,10 +276,10 @@ def measure(kind, n, metric, rows, global_pairs, steps, warmup, rank, world, loc
     # runner.py:104): the chunks share a packed gradient table, expanded (and all-reduced) once per step
     acc = man.table_grad_accumulator(table) if n_chunks > 1 else None
 
-    def run_chunks(get_chunk):
+    def run_chunks(get_chunk, keep=None):
         """one step: every chunk through the public API; one chunk: the collective runs inside its backward on the
         packed gradient table; several chunks: they accumulate in the packed table of `acc`, and acc.finish() runs
-        the collective on it and writes table.grad"""
+        the collective on it and writes table.grad.  keep: a list that receives every chunk's distances"""
         table.grad = None
         total = torch.zeros((), dtype=torch.float64, device=dev)
         for c in range(n_chunks):
@@ -258,6 +290,8 @@ def measure(kind, n, metric, rows, global_pairs, steps, warmup, rank, world, loc
             loss = loss_fn.calculate_loss(gd_c, d * scale)
             loss.backward()
             total += loss.detach()
+            if keep is not None:
+                keep.append(d.detach())
         if acc is not None:
             acc.finish(sync_grad=world > 1)
         return total
@@ -265,8 +299,15 @@ def measure(kind, n, metric, rows, global_pairs, steps, warmup, rank, world, loc
     def resident_chunk(c):
         return idx[c * chunk:(c + 1) * chunk], gd[c * chunk:(c + 1) * chunk]
 
+    last = {}       # with dump_dir: the distances and loss of the latest resident step
+
     def step_resident():
-        return run_chunks(resident_chunk)
+        if dump_dir is None:
+            return run_chunks(resident_chunk)
+        last.clear()
+        last["dist"] = []
+        last["loss"] = run_chunks(resident_chunk, last["dist"])
+        return last["loss"]
 
     host_ms = {}
 
@@ -291,6 +332,11 @@ def measure(kind, n, metric, rows, global_pairs, steps, warmup, rank, world, loc
     time.sleep(0.2)
     ms_total = timed(step_resident, steps, tag="resident")
     clocks = sampler.stop()
+    if dump_dir is not None:
+        if rank == 0:
+            names = dump_outputs(dump_dir, last["dist"], last["loss"], table.grad)
+            print(f"bench: wrote {', '.join(names)} of the last timed step to {dump_dir}", file=sys.stderr)
+        last.clear()
     res = {"value": global_pairs * steps / (ms_total * 1e-3), "ms_per_step": ms_total / steps, "clocks": clocks,
            "host_enqueue_ms_per_step": round(host_ms.get("resident", 0.0), 3),
            "pairs_per_gpu_per_step": b_rank, "chunk_pairs": chunk, "chunks_per_step": n_chunks}
@@ -586,7 +632,8 @@ def run_ours(args):
     warmup = max(args.warmup, 3)
     pcheck = parity_check(rank, world, dev) if world > 1 else None
 
-    res = measure(kind, n, args.metric, rows, global_pairs, args.steps, warmup, rank, world, local, dev)
+    res = measure(kind, n, args.metric, rows, global_pairs, args.steps, warmup, rank, world, local, dev,
+                  dump_dir=args.dump_outputs)
     peaks, peak_src = load_peaks()
     fp64_peak, fp64_clocks = measure_fp64_peak(dev, local)
     roofline = roofline_of(kind, n, res, fp64_peak, fp64_clocks, peaks, peak_src, rows)
@@ -987,7 +1034,14 @@ def main():
     ap.add_argument("--no-extras", action="store_true", help="skip the side measurements (other sizes, epoch times)")
     ap.add_argument("--no-n10", action="store_true", help="skip the n = 10 record")
     ap.add_argument("--cpu-budget", type=float, default=15.0)
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the loss, a sample of the distances and a sample of the table gradient of the last timed "
+                         "step of the headline record as float64 .npy files into DIR")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs is not None and args.impl == "reference":
+        ap.error("--dump-outputs applies to --impl ours")
     if args.impl == "reference":
         run_reference(args)
     else:
