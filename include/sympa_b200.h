@@ -33,7 +33,10 @@ extern "C" {
  *    sympa_workspace_bytes, its layout was never part of the interface).
  * 4: the saved state is packed for EVERY matrix size (so sympa_backward_workspace_bytes is non-zero and
  *    sympa_table_grad_scatter / _expand work for all of them); the packed scatter runs in L2-sized passes
- *    (SYMPA_OPT_SCATTER_PASS_MB); sympa_rsgd_step takes the bounded-domain gradient unsymmetrised. */
+ *    (SYMPA_OPT_SCATTER_PASS_MB); sympa_rsgd_step takes the bounded-domain gradient unsymmetrised.
+ *    Additive since: sympa_average_precision / _workspace_bytes (graph-reconstruction mAP over row blocks of
+ *    the distance matrix).  Callers that need it look the symbol up; the number stays 4 because nothing that
+ *    a version-4 caller relies on changed. */
 #define SYMPA_ABI_VERSION 4
 
 /* manifold kinds: sympa/embeddings.py:144-149 ("upper", "bounded") and :142 ("spd") */
@@ -132,6 +135,24 @@ int sympa_dist_forward(int kind, int n, int metric, int64_t num_pairs,
 int sympa_dist_matrix(int kind, int n, int metric, const double* table, int64_t num_rows,
                       int64_t row_begin, int64_t row_count, const double* wsum_w, double* dist_out,
                       int64_t* idx_workspace, int64_t workspace_pairs, unsigned int* status, void* stream);
+
+/* Graph-reconstruction average precision of rows of a distance matrix (the mAP of the reference's evaluation;
+ * its metric code is not available, so parity with it is unpinned - the definition is restated):
+ *   AP(u) = 1/|N(u)| sum_{v in N(u)} |{v' in N(u) : d(u,v') <= d(u,v)}| / |{w != u : d(u,w) <= d(u,v)}|
+ * which, without ties, is what an argsort-and-scan loop over the row computes (tied nodes rank first).
+ * dist: row-major (row_count x num_cols) block holding rows [row_begin, row_begin + row_count) of the matrix -
+ * what sympa_dist_matrix writes; column row_begin + r (the node itself) is never read as a candidate.
+ * adj_ptr (num_cols + 1) / adj_idx: CSR adjacency of all num_cols nodes, rows free of duplicates; entries equal
+ * to the row's node are ignored, entries outside [0, num_cols) are ignored and set SYMPA_STATUS_BAD_INDEX.
+ * ap_out[r] = AP(row_begin + r), NaN for a row without neighbours or with a NaN distance (which also sets
+ * SYMPA_STATUS_NON_FINITE).  A row's value is bit-identical whatever block, offset or launch shape it comes in.
+ * workspace: device memory, contents irrelevant, of sympa_average_precision_workspace_bytes(row_count,
+ * adj_entries) bytes where adj_entries >= adj_ptr[row_begin + row_count] - adj_ptr[row_begin] (the total entry
+ * count always does); rows whose entries do not fit set SYMPA_STATUS_BAD_INDEX and get NaN. */
+int64_t sympa_average_precision_workspace_bytes(int64_t row_count, int64_t adj_entries);
+int sympa_average_precision(int64_t row_begin, int64_t row_count, int64_t num_cols, const double* dist,
+                            const int64_t* adj_ptr, const int64_t* adj_idx, double* ap_out,
+                            void* workspace, int64_t workspace_bytes, unsigned int* status, void* stream);
 
 /* Backward: replaces autograd through the ~250 torch ops of dist plus the gather backward.
  * grad_dist (num_pairs) is dL/d dist.  Materialised form: grad_z1 / grad_z2 are OVERWRITTEN with

@@ -45,6 +45,8 @@ EXPORTS = (
     "sympa_bounded_rows_to_upper",
     "sympa_bounded_rows_backward",
     "sympa_check_points",
+    "sympa_average_precision_workspace_bytes",
+    "sympa_average_precision",
 )
 
 _lib = None
@@ -110,6 +112,10 @@ def load():
     lib.sympa_bounded_rows_to_upper.argtypes = [I, L, P, P, P, P]
     lib.sympa_bounded_rows_backward.restype = I
     lib.sympa_bounded_rows_backward.argtypes = [I, L, P, P, P, I, P]
+    lib.sympa_average_precision_workspace_bytes.restype = L
+    lib.sympa_average_precision_workspace_bytes.argtypes = [L, L]
+    lib.sympa_average_precision.restype = I
+    lib.sympa_average_precision.argtypes = [L, L, L, P, P, P, P, P, L, P, P]
     _lib = lib
     return lib
 

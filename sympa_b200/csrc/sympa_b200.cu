@@ -5,12 +5,14 @@
 //   scatter_kernel               grad_table[idx] += grad_dist[p] * unit gradient (gather backward,
 //                                replaces the dense index_put of sympa/embeddings.py:34's backward)
 //   wsum_grad_kernel             dL/dw of the learnable wsum metric (sympa/manifolds/metrics.py:103-121)
+//   ap_*_kernel                  average precision of distance-matrix rows (ap_kernels.cuh)
 #include <cuda_runtime.h>
 #include <stdint.h>
 #include <stdio.h>
 
 #include "../../include/sympa_b200.h"
 #include "pair_kernels.cuh"
+#include "ap_kernels.cuh"
 
 namespace sympa {
 
@@ -781,6 +783,45 @@ int sympa_dist_matrix(int kind, int n, int metric, const double* table, int64_t 
     return check_launch();
   }
   return SYMPA_OK;
+}
+
+int64_t sympa_average_precision_workspace_bytes(int64_t row_count, int64_t adj_entries) {
+  if (row_count < 0 || adj_entries < 0) return -1;
+  return (2 * row_count + 2 * adj_entries) * (int64_t)sizeof(double);
+}
+
+int sympa_average_precision(int64_t row_begin, int64_t row_count, int64_t num_cols, const double* dist,
+                            const int64_t* adj_ptr, const int64_t* adj_idx, double* ap_out, void* workspace,
+                            int64_t workspace_bytes, unsigned int* status, void* stream) {
+  if (row_begin < 0 || row_count < 0 || num_cols <= 0 || row_begin + row_count > num_cols) return SYMPA_ERR_BAD_ARG;
+  if (dist == nullptr || adj_ptr == nullptr || ap_out == nullptr || workspace == nullptr) return SYMPA_ERR_BAD_ARG;
+  if (row_count > 0x7FFFFFFFll) return SYMPA_ERR_BAD_ARG;
+  const int64_t cap = workspace_bytes / (int64_t)sizeof(double) / 2 - row_count;
+  if (workspace_bytes < sympa_average_precision_workspace_bytes(row_count, 0) || cap < 0) return SYMPA_ERR_BAD_ARG;
+  if (row_count == 0) return SYMPA_OK;
+  if (adj_idx == nullptr && cap > 0) return SYMPA_ERR_BAD_ARG;
+  cudaStream_t s = (cudaStream_t)stream;
+  int64_t* meta = static_cast<int64_t*>(workspace);
+  double* sorted = reinterpret_cast<double*>(meta + 2 * row_count);
+  unsigned long long* counts = reinterpret_cast<unsigned long long*>(sorted + cap);
+  ap_prepare_kernel<<<(unsigned)row_count, SY_AP_THREADS, 0, s>>>(row_begin, num_cols, dist, adj_ptr, adj_idx, cap, meta,
+                                                                   sorted, counts, status);
+  int rc = check_launch();
+  if (rc) return rc;
+  // split each row over several CTAs until the grid is ~8 CTAs per SM, each CTA keeping >= 16 columns per thread
+  const int64_t want = (int64_t)sm_count() * 8;
+  int64_t splits = (want + row_count - 1) / row_count;
+  const int64_t most = (num_cols + SY_AP_THREADS * 16 - 1) / (SY_AP_THREADS * 16);
+  if (splits > most) splits = most;
+  if (splits < 1) splits = 1;
+  if (row_count * splits > 0x7FFFFFFFll) splits = 1;
+  ap_count_kernel<<<(unsigned)(row_count * splits), SY_AP_THREADS, 0, s>>>(row_begin, num_cols, (int)splits, dist, adj_ptr,
+                                                                           meta, sorted, counts, status);
+  rc = check_launch();
+  if (rc) return rc;
+  ap_finish_kernel<<<(unsigned)((row_count + SY_AP_THREADS - 1) / SY_AP_THREADS), SY_AP_THREADS, 0, s>>>(
+      row_begin, row_count, adj_ptr, meta, sorted, counts, ap_out);
+  return check_launch();
 }
 
 int sympa_dist_backward(int kind, int n, int metric, int64_t num_pairs, const double* grad_dist,

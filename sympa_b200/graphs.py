@@ -59,3 +59,22 @@ def product_cartesian_triplets(branching, height, side, dims):
 
 def product_tree_grid_triplets(branching, height, side, dims):
     return product_cartesian_triplets(branching, height, side, dims)
+
+
+def adjacency_csr(edges, num_nodes):
+    """CSR adjacency (ptr, idx) of the undirected graph with the (E, 2) int64 node pairs `edges` over nodes
+    [0, num_nodes): both directions, duplicates and self loops removed, every row sorted.  ptr has num_nodes + 1
+    entries; the neighbours of u are idx[ptr[u]:ptr[u + 1]].  Returned on the device of `edges`.
+    From triplets: adjacency_csr(ids[gd == 1], n); a tree's edges are (k, parent(k)), e.g. (k, (k - 1) // b)."""
+    edges = torch.as_tensor(edges)
+    if edges.dtype != torch.int64 or edges.dim() != 2 or edges.shape[1] != 2:
+        raise ValueError("edges must be an (E, 2) int64 tensor")
+    if edges.numel() and (int(edges.min()) < 0 or int(edges.max()) >= num_nodes):
+        raise ValueError(f"edge endpoints must lie in [0, {num_nodes})")
+    e = torch.cat((edges, edges.flip(1)))
+    e = e[e[:, 0] != e[:, 1]]
+    key = torch.unique(e[:, 0] * num_nodes + e[:, 1])        # sorted: by source, then by destination
+    src, idx = key // num_nodes, key % num_nodes
+    ptr = torch.zeros(num_nodes + 1, dtype=torch.int64, device=edges.device)
+    ptr[1:] = torch.cumsum(torch.bincount(src, minlength=num_nodes), 0)
+    return ptr, idx.contiguous()

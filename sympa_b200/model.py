@@ -41,6 +41,13 @@ class Model(nn.Module):
                 out[r0:r0 + rc] = self.manifold.dist_matrix(table, r0, rc) * self.get_scale()
             return out
 
+    def mean_average_precision(self, adj, **kw):
+        """Graph-reconstruction mAP of the embedding table against the CSR adjacency `adj`, streamed over row
+        blocks of the distance matrix (see sympa_b200.metrics.mean_average_precision for the keywords)."""
+        from .metrics import mean_average_precision
+        sum_ap, count, _ = mean_average_precision(self.manifold, self.embeddings.embeds, adj, **kw)
+        return sum_ap / max(count, 1)
+
     def get_scale(self):   # model.py:40-41
         return (self.scale / self.scale_coef).clamp_min(0.1)
 

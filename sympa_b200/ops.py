@@ -545,10 +545,11 @@ def distortion_step(kind, metric, table, idx, graph_dist, scale, grad_table, wsu
 _idx_workspace = {}
 
 
-def dist_matrix(kind, metric, table, row_begin=0, row_count=None, wsum_w=None, chunk_pairs=1 << 24):
+def dist_matrix(kind, metric, table, row_begin=0, row_count=None, wsum_w=None, chunk_pairs=1 << 24, out=None):
     """Rows [row_begin, row_begin + row_count) of the all-pairs distance matrix of `table` (forward only,
     zeros on the diagonal): sympa_dist_matrix.  The index workspace (16 bytes per pair of a chunk) is
-    kept per device and reused."""
+    kept per device and reused.  out: an optional contiguous (row_count, N) float64 tensor on the table's
+    device to write into (a streaming caller reuses one block buffer)."""
     lib = _lib.load()
     table = _require(table, "table").detach()
     n = table.shape[-1]
@@ -563,7 +564,11 @@ def dist_matrix(kind, metric, table, row_begin=0, row_count=None, wsum_w=None, c
         wsum_w = None
     dev = table.device
     with torch.cuda.device(dev):
-        out = torch.empty(row_count, rows, dtype=torch.float64, device=dev)
+        if out is None:
+            out = torch.empty(row_count, rows, dtype=torch.float64, device=dev)
+        elif (out.dtype != torch.float64 or out.device != dev or tuple(out.shape) != (row_count, rows)
+              or not out.is_contiguous()):
+            raise ValueError(f"out must be a contiguous float64 ({row_count}, {rows}) tensor on {dev}")
         if row_count == 0 or rows == 0:
             return out
         chunk = max(1, min(chunk_pairs, row_count * rows))
@@ -574,6 +579,51 @@ def dist_matrix(kind, metric, table, row_begin=0, row_count=None, wsum_w=None, c
             _idx_workspace[key] = ws
         _lib.check(lib.sympa_dist_matrix(_lib.KIND[kind], n, _lib.METRIC[metric], _ptr(table), rows, row_begin, row_count,
                                          _ptr(wsum_w), _ptr(out), _ptr(ws), chunk, _ptr(status_word(dev)), _stream()))
+    return out
+
+
+_ap_workspace = {}
+
+
+def average_precision(dist_block, row_begin, adj, out=None):
+    """Graph-reconstruction average precision of rows [row_begin, row_begin + R) of a distance matrix, given as
+    the (R, N) block `dist_block` of those rows (what dist_matrix returns): sympa_average_precision.
+    adj = (ptr, idx): the CSR adjacency of all N nodes on the block's device (graphs.adjacency_csr).  Returns
+    (R,) float64, NaN for a node without neighbours; `out` (R,) to write into.  The workspace (16 bytes per row
+    and per adjacency entry) is kept per device and reused.  Parity with the reference's metric code is
+    unpinned (it is not available): the definition is the one in include/sympa_b200.h."""
+    lib = _lib.load()
+    dist_block = _require(dist_block, "dist_block")
+    if dist_block.dim() != 2:
+        raise ValueError("dist_block must be (rows, N)")
+    ptr, idx = adj
+    ptr = _require(ptr, "adjacency ptr", torch.int64)
+    idx = _require(idx, "adjacency idx", torch.int64)
+    rows, n_cols = dist_block.shape
+    dev = dist_block.device
+    if ptr.device != dev or idx.device != dev:
+        raise ValueError("the adjacency must be on the distance block's device")
+    if ptr.dim() != 1 or ptr.numel() != n_cols + 1 or idx.dim() != 1:
+        raise ValueError(f"adjacency ptr must have N + 1 = {n_cols + 1} entries and idx must be 1-D")
+    if row_begin < 0 or row_begin + rows > n_cols:
+        raise ValueError("row range outside the matrix")
+    if out is None:
+        out = torch.empty(rows, dtype=torch.float64, device=dev)
+    elif out.dtype != torch.float64 or out.device != dev or tuple(out.shape) != (rows,) or not out.is_contiguous():
+        raise ValueError(f"out must be a contiguous float64 ({rows},) tensor on {dev}")
+    if rows == 0:
+        return out
+    with torch.cuda.device(dev):
+        nbytes = lib.sympa_average_precision_workspace_bytes(rows, idx.numel())
+        key = (dev.type, dev.index if dev.index is not None else torch.cuda.current_device())
+        ws = _ap_workspace.get(key)
+        if ws is None or ws.numel() * 8 < nbytes:
+            ws = torch.empty(nbytes // 8, dtype=torch.float64, device=dev)
+            _ap_workspace[key] = ws
+        if idx.numel() == 0:
+            idx = torch.zeros(1, dtype=torch.int64, device=dev)     # no entries: any valid pointer
+        _lib.check(lib.sympa_average_precision(row_begin, rows, n_cols, _ptr(dist_block), _ptr(ptr), _ptr(idx), _ptr(out),
+                                               _ptr(ws), ws.numel() * 8, _ptr(status_word(dev)), _stream()))
     return out
 
 
