@@ -35,8 +35,10 @@ extern "C" {
  *    sympa_table_grad_scatter / _expand work for all of them); the packed scatter runs in L2-sized passes
  *    (SYMPA_OPT_SCATTER_PASS_MB); sympa_rsgd_step takes the bounded-domain gradient unsymmetrised.
  *    Additive since: sympa_average_precision / _workspace_bytes (graph-reconstruction mAP over row blocks of
- *    the distance matrix).  Callers that need it look the symbol up; the number stays 4 because nothing that
- *    a version-4 caller relies on changed. */
+ *    the distance matrix); sympa_hop_distances / _workspace_bytes and sympa_distortion_rows (graph hop
+ *    distances by breadth-first search, graph-reconstruction distortion over the same row blocks).  Callers
+ *    that need them look the symbols up; the number stays 4 because nothing that a version-4 caller relies on
+ *    changed. */
 #define SYMPA_ABI_VERSION 4
 
 /* manifold kinds: sympa/embeddings.py:144-149 ("upper", "bounded") and :142 ("spd") */
@@ -153,6 +155,38 @@ int64_t sympa_average_precision_workspace_bytes(int64_t row_count, int64_t adj_e
 int sympa_average_precision(int64_t row_begin, int64_t row_count, int64_t num_cols, const double* dist,
                             const int64_t* adj_ptr, const int64_t* adj_idx, double* ap_out,
                             void* workspace, int64_t workspace_bytes, unsigned int* status, void* stream);
+
+/* Hop distances of the undirected graph given by the CSR adjacency adj_ptr (num_nodes + 1) / adj_idx (valid
+ * pointers: non-decreasing, every entry of [adj_ptr[0], adj_ptr[num_nodes]) readable), by breadth-first search
+ * from every source of rows [row_begin, row_begin + row_count).  hops_out: row-major (row_count x num_nodes)
+ * int32, entry [r][v] = hop distance from row_begin + r to v, 0 on the diagonal, -1 where v is unreachable.
+ * Entries outside [0, num_nodes) are skipped and set SYMPA_STATUS_BAD_INDEX.  The output is identical on every
+ * run and for every block or offset (breadth-first distances are unique; only the queue order varies).
+ * workspace: device memory, contents irrelevant, of sympa_hop_distances_workspace_bytes(num_nodes) bytes - one
+ * queue of num_nodes int32 per resident CTA of a persistent grid, so it does not grow with row_count.  Work per
+ * source is O(num_nodes + entries) with one CTA barrier per BFS level. */
+int64_t sympa_hop_distances_workspace_bytes(int64_t num_nodes);
+int sympa_hop_distances(int64_t row_begin, int64_t row_count, int64_t num_nodes, const int64_t* adj_ptr,
+                        const int64_t* adj_idx, int32_t* hops_out, void* workspace, int64_t workspace_bytes,
+                        unsigned int* status, void* stream);
+
+/* Graph-reconstruction distortion of rows of a distance matrix (the reference's evaluation reports the average;
+ * its metric code is not available, so parity with it is unpinned - the definition is restated).  With g(u, w)
+ * the hop distance, s the model scale and d(u, w) row u, column w of the distance matrix, over the pairs u < w
+ * connected in the graph (the reference's triplets):
+ *   delta(u, w) = |s d(u, w) - g(u, w)| / g(u, w)
+ *   average distortion    = mean of delta over all pairs
+ *   worst-case distortion = max(s d / g) / min(s d / g) over all pairs
+ * dist: the (row_count x num_cols) float64 block of rows [row_begin, row_begin + row_count) (sympa_dist_matrix),
+ * hops: the int32 block of the same rows (sympa_hop_distances).  For row u = row_begin + r, over the columns
+ * w > u with hops >= 1: sum_out[r] = sum of delta, count_out[r] = the number of pairs, max_out[r] / min_out[r] =
+ * the extremes of s d / g (-inf / +inf for a row without pairs).  A NaN among the row's scaled distances makes
+ * all three float outputs NaN and sets SYMPA_STATUS_NON_FINITE.  Each row is summed in one fixed order: its
+ * values are bit-identical whatever block, offset or shard it comes in.  Reads 12 bytes per entry of the
+ * row's upper part. */
+int sympa_distortion_rows(int64_t row_begin, int64_t row_count, int64_t num_cols, const double* dist, const int32_t* hops,
+                          double scale, double* sum_out, int64_t* count_out, double* max_out, double* min_out,
+                          unsigned int* status, void* stream);
 
 /* Backward: replaces autograd through the ~250 torch ops of dist plus the gather backward.
  * grad_dist (num_pairs) is dL/d dist.  Materialised form: grad_z1 / grad_z2 are OVERWRITTEN with

@@ -47,6 +47,9 @@ EXPORTS = (
     "sympa_check_points",
     "sympa_average_precision_workspace_bytes",
     "sympa_average_precision",
+    "sympa_hop_distances_workspace_bytes",
+    "sympa_hop_distances",
+    "sympa_distortion_rows",
 )
 
 _lib = None
@@ -116,6 +119,12 @@ def load():
     lib.sympa_average_precision_workspace_bytes.argtypes = [L, L]
     lib.sympa_average_precision.restype = I
     lib.sympa_average_precision.argtypes = [L, L, L, P, P, P, P, P, L, P, P]
+    lib.sympa_hop_distances_workspace_bytes.restype = L
+    lib.sympa_hop_distances_workspace_bytes.argtypes = [L]
+    lib.sympa_hop_distances.restype = I
+    lib.sympa_hop_distances.argtypes = [L, L, L, P, P, P, P, L, P, P]
+    lib.sympa_distortion_rows.restype = I
+    lib.sympa_distortion_rows.argtypes = [L, L, L, P, P, D, P, P, P, P, P, P]
     _lib = lib
     return lib
 

@@ -6,6 +6,8 @@
 //                                replaces the dense index_put of sympa/embeddings.py:34's backward)
 //   wsum_grad_kernel             dL/dw of the learnable wsum metric (sympa/manifolds/metrics.py:103-121)
 //   ap_*_kernel                  average precision of distance-matrix rows (ap_kernels.cuh)
+//   hop_bfs_kernel               graph hop distances of a block of source rows (hop_kernels.cuh)
+//   distortion_rows_kernel       graph-reconstruction distortion of distance-matrix rows (hop_kernels.cuh)
 #include <cuda_runtime.h>
 #include <stdint.h>
 #include <stdio.h>
@@ -13,6 +15,7 @@
 #include "../../include/sympa_b200.h"
 #include "pair_kernels.cuh"
 #include "ap_kernels.cuh"
+#include "hop_kernels.cuh"
 
 namespace sympa {
 
@@ -821,6 +824,51 @@ int sympa_average_precision(int64_t row_begin, int64_t row_count, int64_t num_co
   if (rc) return rc;
   ap_finish_kernel<<<(unsigned)((row_count + SY_AP_THREADS - 1) / SY_AP_THREADS), SY_AP_THREADS, 0, s>>>(
       row_begin, row_count, adj_ptr, meta, sorted, counts, ap_out);
+  return check_launch();
+}
+
+int64_t sympa_hop_distances_workspace_bytes(int64_t num_nodes) {
+  if (num_nodes < 0 || num_nodes > 0x7FFFFFFFll) return -1;
+  return SY_HOP_HEADER_BYTES + (int64_t)SY_HOP_CTAS_PER_SM * sm_count() * num_nodes * (int64_t)sizeof(int);
+}
+
+int sympa_hop_distances(int64_t row_begin, int64_t row_count, int64_t num_nodes, const int64_t* adj_ptr,
+                        const int64_t* adj_idx, int32_t* hops_out, void* workspace, int64_t workspace_bytes,
+                        unsigned int* status, void* stream) {
+  if (row_begin < 0 || row_count < 0 || num_nodes < 0 || num_nodes > 0x7FFFFFFFll || row_begin + row_count > num_nodes)
+    return SYMPA_ERR_BAD_ARG;
+  if (row_count == 0) return SYMPA_OK;
+  if (adj_ptr == nullptr || adj_idx == nullptr || hops_out == nullptr || workspace == nullptr) return SYMPA_ERR_BAD_ARG;
+  if (workspace_bytes < sympa_hop_distances_workspace_bytes(num_nodes)) return SYMPA_ERR_BAD_ARG;
+  cudaStream_t s = (cudaStream_t)stream;
+  unsigned int* ticket = static_cast<unsigned int*>(workspace);
+  int* queues = reinterpret_cast<int*>(static_cast<char*>(workspace) + SY_HOP_HEADER_BYTES);
+  if (cudaMemsetAsync(ticket, 0, sizeof(unsigned int), s) != cudaSuccess) return check_launch();
+  int64_t grid = (int64_t)SY_HOP_CTAS_PER_SM * sm_count();
+  if (grid > row_count) grid = row_count;
+  const int64_t visited_bytes = (num_nodes + 31) / 32 * (int64_t)sizeof(unsigned int);
+  static_assert(SY_HOP_SMEM_VISITED_BYTES <= 48 * 1024 - 256,
+                "the bitmap must leave room for the kernel's static shared memory under the 48 KB default");
+  if (visited_bytes <= SY_HOP_SMEM_VISITED_BYTES)
+    hop_bfs_kernel<true><<<(unsigned)grid, SY_HOP_THREADS, (size_t)visited_bytes, s>>>(
+        row_begin, (int)row_count, (int)num_nodes, adj_ptr, adj_idx, hops_out, queues, ticket, status);
+  else
+    hop_bfs_kernel<false><<<(unsigned)grid, SY_HOP_THREADS, 0, s>>>(row_begin, (int)row_count, (int)num_nodes, adj_ptr,
+                                                                    adj_idx, hops_out, queues, ticket, status);
+  return check_launch();
+}
+
+int sympa_distortion_rows(int64_t row_begin, int64_t row_count, int64_t num_cols, const double* dist, const int32_t* hops,
+                          double scale, double* sum_out, int64_t* count_out, double* max_out, double* min_out,
+                          unsigned int* status, void* stream) {
+  if (row_begin < 0 || row_count < 0 || num_cols < 0 || row_begin + row_count > num_cols || row_count > 0x7FFFFFFFll)
+    return SYMPA_ERR_BAD_ARG;
+  if (row_count == 0) return SYMPA_OK;
+  if (dist == nullptr || hops == nullptr || sum_out == nullptr || count_out == nullptr || max_out == nullptr ||
+      min_out == nullptr)
+    return SYMPA_ERR_BAD_ARG;
+  distortion_rows_kernel<<<(unsigned)row_count, SY_DISTORTION_THREADS, 0, (cudaStream_t)stream>>>(
+      row_begin, num_cols, dist, hops, scale, sum_out, count_out, max_out, min_out, status);
   return check_launch();
 }
 

@@ -78,3 +78,35 @@ def adjacency_csr(edges, num_nodes):
     ptr = torch.zeros(num_nodes + 1, dtype=torch.int64, device=edges.device)
     ptr[1:] = torch.cumsum(torch.bincount(src, minlength=num_nodes), 0)
     return ptr, idx.contiguous()
+
+
+def shortest_path_triplets(adj, block_bytes=1 << 30):
+    """(src, dst, distance) triplets of every pair i < j joined by a path in the undirected graph adj = (ptr, idx)
+    (adjacency_csr), distance = hop count: the format and order of the generators above, for any graph - what
+    preprocess.py:114 gets from networkit's all-pairs shortest paths.  Hop distances come from breadth-first search
+    on the GPU (ops.hop_distances) in blocks of max(1, block_bytes // (4 N)) source rows, on adj's device when it
+    is a CUDA device and on the current one otherwise; the result is returned on adj's device.  Meant for graphs
+    whose triplets fit in memory (24 bytes per pair)."""
+    from . import ops
+
+    ptr, idx = adj
+    out_dev = torch.as_tensor(ptr).device
+    dev = out_dev if out_dev.type == "cuda" else torch.device("cuda", torch.cuda.current_device())
+    ptr = torch.as_tensor(ptr, dtype=torch.int64).to(dev).contiguous()
+    idx = torch.as_tensor(idx, dtype=torch.int64).to(dev).contiguous()
+    n = ptr.numel() - 1
+    block = max(1, min(block_bytes // (4 * max(n, 1)), max(n, 1)))
+    cols = torch.arange(n, device=dev)
+    ids, dist = [], []
+    for r0 in range(0, n, block):
+        rc = min(block, n - r0)
+        h = ops.hop_distances((ptr, idx), r0, rc)
+        keep = (h > 0) & (cols[None, :] > torch.arange(r0, r0 + rc, device=dev)[:, None])
+        rc_idx = keep.nonzero()
+        rc_idx[:, 0] += r0
+        ids.append(rc_idx.to(out_dev))
+        dist.append(h[keep].double().to(out_dev))
+    ops.check_status(dev)
+    if not ids:
+        return torch.zeros(0, 2, dtype=torch.int64, device=out_dev), torch.zeros(0, dtype=torch.float64, device=out_dev), n
+    return torch.cat(ids).contiguous(), torch.cat(dist), n

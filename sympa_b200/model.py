@@ -48,6 +48,25 @@ class Model(nn.Module):
         sum_ap, count, _ = mean_average_precision(self.manifold, self.embeddings.embeds, adj, **kw)
         return sum_ap / max(count, 1)
 
+    def average_distortion(self, adj, **kw):
+        """Average graph-reconstruction distortion of the embedding table, distances scaled by get_scale(), against
+        the hop distances of the CSR adjacency `adj`, streamed over row blocks of the distance matrix (see
+        sympa_b200.metrics.average_distortion for the keywords)."""
+        from .metrics import average_distortion
+        total, count, _, _, _ = average_distortion(self.manifold, self.embeddings.embeds, adj, scale=self._eval_scale(), **kw)
+        return total / count if count else float("nan")
+
+    def evaluate(self, adj, **kw):
+        """(average distortion, mAP) - the pair Runner.evaluate (sympa/runner.py:124-154) reports - in one pass over
+        row blocks of the distance matrix (see sympa_b200.metrics.evaluate for the keywords)."""
+        from .metrics import evaluate
+        r = evaluate(self.manifold, self.embeddings.embeds, adj, scale=self._eval_scale(), **kw)
+        return r.average_distortion, r.mean_ap
+
+    def _eval_scale(self):
+        with torch.no_grad():
+            return float(self.get_scale().item())
+
     def get_scale(self):   # model.py:40-41
         return (self.scale / self.scale_coef).clamp_min(0.1)
 

@@ -3,6 +3,7 @@
 PyTorch is used for device memory, streams and autograd plumbing only; all arithmetic of
 `dist` happens in libsympa_b200.so.  Tensors must be CUDA float64 and contiguous.
 """
+import collections
 import os
 
 import torch
@@ -624,6 +625,90 @@ def average_precision(dist_block, row_begin, adj, out=None):
             idx = torch.zeros(1, dtype=torch.int64, device=dev)     # no entries: any valid pointer
         _lib.check(lib.sympa_average_precision(row_begin, rows, n_cols, _ptr(dist_block), _ptr(ptr), _ptr(idx), _ptr(out),
                                                _ptr(ws), ws.numel() * 8, _ptr(status_word(dev)), _stream()))
+    return out
+
+
+_hop_workspace = {}
+
+
+def hop_distances(adj, row_begin, row_count, out=None):
+    """Hop distances from the sources [row_begin, row_begin + row_count) to every node of the undirected graph
+    adj = (ptr, idx) (the CSR adjacency of graphs.adjacency_csr, on a CUDA device), by breadth-first search on
+    the device: sympa_hop_distances.  Returns the (row_count, N) int32 block, 0 on the diagonal and -1 where a
+    node is unreachable; `out` to write into.  The workspace (one queue of N int32 per resident CTA, independent
+    of row_count) is kept per device and reused."""
+    lib = _lib.load()
+    ptr, idx = adj
+    ptr = _require(ptr, "adjacency ptr", torch.int64)
+    idx = _require(idx, "adjacency idx", torch.int64)
+    dev = ptr.device
+    if idx.device != dev:
+        raise ValueError("adjacency ptr and idx must be on the same device")
+    if ptr.dim() != 1 or ptr.numel() < 1 or idx.dim() != 1:
+        raise ValueError("adjacency ptr must be 1-D with N + 1 entries and idx must be 1-D")
+    n_nodes = ptr.numel() - 1
+    if row_begin < 0 or row_count < 0 or row_begin + row_count > n_nodes:
+        raise ValueError("row range outside the graph")
+    if out is None:
+        out = torch.empty(row_count, n_nodes, dtype=torch.int32, device=dev)
+    elif (out.dtype != torch.int32 or out.device != dev or tuple(out.shape) != (row_count, n_nodes)
+          or not out.is_contiguous()):
+        raise ValueError(f"out must be a contiguous int32 ({row_count}, {n_nodes}) tensor on {dev}")
+    if row_count == 0:
+        return out
+    with torch.cuda.device(dev):
+        nbytes = lib.sympa_hop_distances_workspace_bytes(n_nodes)
+        if nbytes < 0:
+            raise ValueError(f"graphs of {n_nodes} nodes are not supported (int32 node ids)")
+        key = (dev.type, dev.index if dev.index is not None else torch.cuda.current_device())
+        ws = _hop_workspace.get(key)
+        if ws is None or ws.numel() * 8 < nbytes:
+            ws = torch.empty((nbytes + 7) // 8, dtype=torch.float64, device=dev)
+            _hop_workspace[key] = ws
+        if idx.numel() == 0:
+            idx = torch.zeros(1, dtype=torch.int64, device=dev)     # no entries: any valid pointer
+        _lib.check(lib.sympa_hop_distances(row_begin, row_count, n_nodes, _ptr(ptr), _ptr(idx), _ptr(out), _ptr(ws),
+                                           ws.numel() * 8, _ptr(status_word(dev)), _stream()))
+    return out
+
+
+DistortionRows = collections.namedtuple("DistortionRows", "sum count max min")
+DistortionRows.__doc__ = """Per-row distortion terms (sympa_distortion_rows): over the pairs (u, w > u) connected in the
+graph, sum of |s d - g| / g (float64), the number of pairs (int64) and the extremes of s d / g (float64;
+-inf / +inf for a row without pairs, NaN for a row with a NaN distance)."""
+
+
+def distortion_rows(dist_block, hop_block, row_begin, scale, out=None):
+    """Graph-reconstruction distortion terms of rows [row_begin, row_begin + R) of a distance matrix, from the
+    (R, N) float64 block `dist_block` of those rows (dist_matrix) and the (R, N) int32 hop block of the same
+    rows (hop_distances): sympa_distortion_rows.  `scale` multiplies every distance (the model scale).
+    Returns a DistortionRows of (R,) tensors; `out` a DistortionRows to write into.  A row's values are
+    bit-identical whatever block it comes in.  Parity with the reference's metric code is unpinned (it is not
+    available): the definition is the one in include/sympa_b200.h."""
+    lib = _lib.load()
+    dist_block = _require(dist_block, "dist_block")
+    hop_block = _require(hop_block, "hop_block", torch.int32)
+    if dist_block.dim() != 2:
+        raise ValueError("dist_block must be (rows, N)")
+    rows, n_cols = dist_block.shape
+    dev = dist_block.device
+    if hop_block.device != dev or tuple(hop_block.shape) != (rows, n_cols):
+        raise ValueError(f"hop_block must be ({rows}, {n_cols}) on {dev}")
+    if row_begin < 0 or row_begin + rows > n_cols:
+        raise ValueError("row range outside the matrix")
+    dtypes = DistortionRows(torch.float64, torch.int64, torch.float64, torch.float64)
+    if out is None:
+        out = DistortionRows(*(torch.empty(rows, dtype=t, device=dev) for t in dtypes))
+    else:
+        out = DistortionRows(*out)
+        for o, t in zip(out, dtypes):
+            if o.dtype != t or o.device != dev or tuple(o.shape) != (rows,) or not o.is_contiguous():
+                raise ValueError(f"out must hold contiguous ({rows},) tensors on {dev} of dtypes {tuple(dtypes)}")
+    if rows == 0:
+        return out
+    with torch.cuda.device(dev):
+        _lib.check(lib.sympa_distortion_rows(row_begin, rows, n_cols, _ptr(dist_block), _ptr(hop_block), float(scale),
+                                             *(_ptr(o) for o in out), _ptr(status_word(dev)), _stream()))
     return out
 
 
