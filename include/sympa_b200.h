@@ -36,7 +36,9 @@ extern "C" {
  *    (SYMPA_OPT_SCATTER_PASS_MB); sympa_rsgd_step takes the bounded-domain gradient unsymmetrised.
  *    Additive since: sympa_average_precision / _workspace_bytes (graph-reconstruction mAP over row blocks of
  *    the distance matrix); sympa_hop_distances / _workspace_bytes and sympa_distortion_rows (graph hop
- *    distances by breadth-first search, graph-reconstruction distortion over the same row blocks).  Callers
+ *    distances by breadth-first search, graph-reconstruction distortion over the same row blocks);
+ *    sympa_sample_pairs / _workspace_bytes and SYMPA_STATUS_NO_PAIR (training pairs and their hop distances
+ *    sampled by breadth-first search from a list of sources).  Callers
  *    that need them look the symbols up; the number stays 4 because nothing that a version-4 caller relies on
  *    changed. */
 #define SYMPA_ABI_VERSION 4
@@ -61,6 +63,7 @@ enum {
 #define SYMPA_STATUS_NO_CONVERGE 4u       /* Jacobi sweep cap reached */
 #define SYMPA_STATUS_NON_FINITE 8u
 #define SYMPA_STATUS_BAD_INDEX 16u        /* idx outside [0, num_rows) - the pair is skipped */
+#define SYMPA_STATUS_NO_PAIR 32u          /* a sampling source reaches no other node (sympa_sample_pairs) */
 
 int sympa_version(void);
 const char* sympa_error_string(int code);
@@ -169,6 +172,30 @@ int64_t sympa_hop_distances_workspace_bytes(int64_t num_nodes);
 int sympa_hop_distances(int64_t row_begin, int64_t row_count, int64_t num_nodes, const int64_t* adj_ptr,
                         const int64_t* adj_idx, int32_t* hops_out, void* workspace, int64_t workspace_bytes,
                         unsigned int* status, void* stream);
+
+/* Training pairs sampled from the undirected graph of the CSR adjacency adj_ptr (num_nodes + 1) / adj_idx (as for
+ * sympa_hop_distances), K = pairs_per_source per source, without an N-wide row per source ever reaching the output.
+ * With mix the SplitMix64 finalizer (all arithmetic mod 2^64)
+ *   mix(x):  x += 0x9E3779B97F4A7C15;  x = (x ^ (x >> 30)) * 0xBF58476D1CE4E5B9;
+ *            x = (x ^ (x >> 27)) * 0x94D049BB133111EB;  x ^= x >> 31
+ *   h(seed, epoch, tag, a, b) = mix(mix(mix(mix(mix(seed) ^ epoch) ^ tag) ^ a) ^ b)
+ * and R(u) the nodes reachable from u, c = |R(u)| - 1: draw k = 0 .. K-1 of source u is the r-th node (0-based) of
+ * R(u) \ {u} in ascending node id, r = floor(h(seed, epoch, 0, u, k) * c / 2^64), with its hop distance g >= 1.
+ * Draws are uniform with replacement (bias at most c / 2^64) and depend on nothing else: not the queue order, the
+ * launch shape, the source's position in the list or the other sources.
+ * sources: num_sources int64 node ids.  idx_out: (num_sources * K, 2) int64 [u, dst]; dist_out: (num_sources * K)
+ * float64 g; the pairs of sources[i] are rows i*K .. i*K + K-1, k ascending.  A source outside [0, num_nodes) sets
+ * SYMPA_STATUS_BAD_INDEX, one that reaches no other node SYMPA_STATUS_NO_PAIR; both get K pairs (u, u) at distance
+ * 0.  Adjacency entries outside [0, num_nodes) are skipped and set SYMPA_STATUS_BAD_INDEX.
+ * workspace: device memory, contents irrelevant, of sympa_sample_pairs_workspace_bytes(num_nodes) bytes - per
+ * resident CTA of a persistent grid a queue, a row of hop distances and the reached set with its popcount prefixes,
+ * about 8.25 bytes per node; it grows with neither num_sources nor K.  Work per source is one breadth-first search
+ * (O(num_nodes + entries)) plus O(K log num_nodes). */
+int64_t sympa_sample_pairs_workspace_bytes(int64_t num_nodes);
+int sympa_sample_pairs(int64_t num_nodes, const int64_t* adj_ptr, const int64_t* adj_idx, int64_t num_sources,
+                       const int64_t* sources, int64_t pairs_per_source, uint64_t seed, uint64_t epoch,
+                       int64_t* idx_out, double* dist_out, void* workspace, int64_t workspace_bytes,
+                       unsigned int* status, void* stream);
 
 /* Graph-reconstruction distortion of rows of a distance matrix (the reference's evaluation reports the average;
  * its metric code is not available, so parity with it is unpinned - the definition is restated).  With g(u, w)

@@ -18,6 +18,7 @@ STATUS_BITS = {
     4: "Jacobi sweep cap reached",
     8: "non-finite distance",
     16: "table index out of range",
+    32: "a sampling source reaches no other node",
 }
 
 EXPORTS = (
@@ -50,6 +51,8 @@ EXPORTS = (
     "sympa_hop_distances_workspace_bytes",
     "sympa_hop_distances",
     "sympa_distortion_rows",
+    "sympa_sample_pairs_workspace_bytes",
+    "sympa_sample_pairs",
 )
 
 _lib = None
@@ -125,6 +128,10 @@ def load():
     lib.sympa_hop_distances.argtypes = [L, L, L, P, P, P, P, L, P, P]
     lib.sympa_distortion_rows.restype = I
     lib.sympa_distortion_rows.argtypes = [L, L, L, P, P, D, P, P, P, P, P, P]
+    lib.sympa_sample_pairs_workspace_bytes.restype = L
+    lib.sympa_sample_pairs_workspace_bytes.argtypes = [L]
+    lib.sympa_sample_pairs.restype = I
+    lib.sympa_sample_pairs.argtypes = [L, P, P, L, P, L, ctypes.c_uint64, ctypes.c_uint64, P, P, P, L, P, P]
     _lib = lib
     return lib
 

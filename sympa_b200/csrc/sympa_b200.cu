@@ -7,6 +7,7 @@
 //   wsum_grad_kernel             dL/dw of the learnable wsum metric (sympa/manifolds/metrics.py:103-121)
 //   ap_*_kernel                  average precision of distance-matrix rows (ap_kernels.cuh)
 //   hop_bfs_kernel               graph hop distances of a block of source rows (hop_kernels.cuh)
+//   sample_pairs_kernel          training pairs and their hop distances sampled per source (hop_kernels.cuh)
 //   distortion_rows_kernel       graph-reconstruction distortion of distance-matrix rows (hop_kernels.cuh)
 #include <cuda_runtime.h>
 #include <stdint.h>
@@ -855,6 +856,41 @@ int sympa_hop_distances(int64_t row_begin, int64_t row_count, int64_t num_nodes,
   else
     hop_bfs_kernel<false><<<(unsigned)grid, SY_HOP_THREADS, 0, s>>>(row_begin, (int)row_count, (int)num_nodes, adj_ptr,
                                                                     adj_idx, hops_out, queues, ticket, status);
+  return check_launch();
+}
+
+int64_t sympa_sample_pairs_workspace_bytes(int64_t num_nodes) {
+  if (num_nodes < 0 || num_nodes > 0x7FFFFFFFll) return -1;
+  return SY_HOP_HEADER_BYTES + (int64_t)SY_HOP_CTAS_PER_SM * sm_count() * sample_slice_ints(num_nodes) * (int64_t)sizeof(int);
+}
+
+int sympa_sample_pairs(int64_t num_nodes, const int64_t* adj_ptr, const int64_t* adj_idx, int64_t num_sources,
+                       const int64_t* sources, int64_t pairs_per_source, uint64_t seed, uint64_t epoch,
+                       int64_t* idx_out, double* dist_out, void* workspace, int64_t workspace_bytes,
+                       unsigned int* status, void* stream) {
+  if (num_nodes < 0 || num_nodes > 0x7FFFFFFFll || num_sources < 0 || num_sources > 0x7FFFFFFFll || pairs_per_source < 0)
+    return SYMPA_ERR_BAD_ARG;
+  if (num_sources > 0 && pairs_per_source > INT64_MAX / 2 / num_sources) return SYMPA_ERR_BAD_ARG;
+  if (num_sources == 0 || pairs_per_source == 0) return SYMPA_OK;
+  if (adj_ptr == nullptr || adj_idx == nullptr || sources == nullptr || idx_out == nullptr || dist_out == nullptr ||
+      workspace == nullptr)
+    return SYMPA_ERR_BAD_ARG;
+  if (workspace_bytes < sympa_sample_pairs_workspace_bytes(num_nodes)) return SYMPA_ERR_BAD_ARG;
+  cudaStream_t s = (cudaStream_t)stream;
+  unsigned int* ticket = static_cast<unsigned int*>(workspace);
+  int* slices = reinterpret_cast<int*>(static_cast<char*>(workspace) + SY_HOP_HEADER_BYTES);
+  if (cudaMemsetAsync(ticket, 0, sizeof(unsigned int), s) != cudaSuccess) return check_launch();
+  int64_t grid = (int64_t)SY_HOP_CTAS_PER_SM * sm_count();
+  if (grid > num_sources) grid = num_sources;
+  const int64_t visited_bytes = (num_nodes + 31) / 32 * (int64_t)sizeof(unsigned int);
+  if (visited_bytes <= SY_HOP_SMEM_VISITED_BYTES)
+    sample_pairs_kernel<true><<<(unsigned)grid, SY_HOP_THREADS, (size_t)visited_bytes, s>>>(
+        (int)num_sources, (int)num_nodes, adj_ptr, adj_idx, sources, pairs_per_source, seed, epoch, idx_out, dist_out,
+        slices, ticket, status);
+  else
+    sample_pairs_kernel<false><<<(unsigned)grid, SY_HOP_THREADS, 0, s>>>(
+        (int)num_sources, (int)num_nodes, adj_ptr, adj_idx, sources, pairs_per_source, seed, epoch, idx_out, dist_out,
+        slices, ticket, status);
   return check_launch();
 }
 

@@ -672,6 +672,65 @@ def hop_distances(adj, row_begin, row_count, out=None):
     return out
 
 
+_sample_workspace = {}
+
+
+def sample_pairs(adj, sources, k, seed, epoch, out=None):
+    """K = k training pairs per source of the undirected graph adj = (ptr, idx) (graphs.adjacency_csr, on a CUDA
+    device), drawn uniformly with replacement from the nodes each source reaches, with their hop distances, by
+    breadth-first search on the device: sympa_sample_pairs.  The draws are a fixed function of (seed, epoch, source,
+    draw number), defined in include/sympa_b200.h.  sources: 1-D int64 node ids on adj's device.  Returns
+    (src_dst_ids (S k, 2) int64, graph_distances (S k,) float64), the pairs of sources[i] in rows i k .. i k + k - 1:
+    the tensors the trainers take.  out = (ids, gd) to write into.  A source outside [0, N) sets the status bit of
+    an out-of-range index, one that reaches no other node its own bit (check_status); both get k pairs (u, u) at
+    distance 0.  The workspace (about 8.25 bytes per node per resident CTA, independent of S and k) is kept per
+    device and reused."""
+    lib = _lib.load()
+    ptr, idx = adj
+    ptr = _require(ptr, "adjacency ptr", torch.int64)
+    idx = _require(idx, "adjacency idx", torch.int64)
+    sources = _require(sources, "sources", torch.int64)
+    dev = ptr.device
+    if idx.device != dev or sources.device != dev:
+        raise ValueError("adjacency ptr, idx and sources must be on the same device")
+    if ptr.dim() != 1 or ptr.numel() < 1 or idx.dim() != 1:
+        raise ValueError("adjacency ptr must be 1-D with N + 1 entries and idx must be 1-D")
+    if sources.dim() != 1:
+        raise ValueError("sources must be 1-D")
+    k, seed, epoch = int(k), int(seed), int(epoch)
+    if k < 0:
+        raise ValueError("k must be >= 0")
+    if not (0 <= seed < 1 << 64 and 0 <= epoch < 1 << 64):
+        raise ValueError("seed and epoch must lie in [0, 2^64)")
+    n_nodes, s = ptr.numel() - 1, sources.numel()
+    if s >= 1 << 31:
+        raise ValueError("at most 2^31 - 1 sources per call")
+    if n_nodes >= 1 << 31:
+        raise ValueError(f"graphs of {n_nodes} nodes are not supported (int32 node ids)")
+    if out is None:
+        out = (torch.empty(s * k, 2, dtype=torch.int64, device=dev), torch.empty(s * k, dtype=torch.float64, device=dev))
+    else:
+        ids, gd = out
+        if (ids.dtype != torch.int64 or ids.device != dev or tuple(ids.shape) != (s * k, 2) or not ids.is_contiguous()
+                or gd.dtype != torch.float64 or gd.device != dev or tuple(gd.shape) != (s * k,) or not gd.is_contiguous()):
+            raise ValueError(f"out must be contiguous int64 ({s * k}, 2) and float64 ({s * k},) tensors on {dev}")
+        out = (ids, gd)
+    if s * k == 0:
+        return out
+    with torch.cuda.device(dev):
+        nbytes = lib.sympa_sample_pairs_workspace_bytes(n_nodes)
+        key = (dev.type, dev.index if dev.index is not None else torch.cuda.current_device())
+        ws = _sample_workspace.get(key)
+        if ws is None or ws.numel() * 8 < nbytes:
+            ws = torch.empty((nbytes + 7) // 8, dtype=torch.float64, device=dev)
+            _sample_workspace[key] = ws
+        if idx.numel() == 0:
+            idx = torch.zeros(1, dtype=torch.int64, device=dev)     # no entries: any valid pointer
+        _lib.check(lib.sympa_sample_pairs(n_nodes, _ptr(ptr), _ptr(idx), s, _ptr(sources), k, seed, epoch, _ptr(out[0]),
+                                          _ptr(out[1]), _ptr(ws), ws.numel() * 8, _ptr(status_word(dev)), _stream()))
+    return out
+
+
 DistortionRows = collections.namedtuple("DistortionRows", "sum count max min")
 DistortionRows.__doc__ = """Per-row distortion terms (sympa_distortion_rows): over the pairs (u, w > u) connected in the
 graph, sum of |s d - g| / g (float64), the number of pairs (int64) and the extremes of s d / g (float64;

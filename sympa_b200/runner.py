@@ -9,7 +9,7 @@ from .losses import AverageDistortionLoss
 
 
 def train_epoch(model, optimizer, src_dst_ids, graph_distances, batch_size, max_grad_norm=50.0, grad_accum_steps=1,
-                world_size=1, rank=0, epoch=0, shuffle=True, sync_stats=True, device_shuffle=False):
+                world_size=1, rank=0, epoch=0, shuffle=True, sync_stats=True, device_shuffle=False, presharded=False):
     """One pass over the training triplets (runner.py:90-122).
 
     src_dst_ids (T, 2) int64 and graph_distances (T,) live on the device (train.py:95-96).  Each rank
@@ -18,12 +18,14 @@ def train_epoch(model, optimizer, src_dst_ids, graph_distances, batch_size, max_
     (what DistributedDataParallel does, train.py:59) - the one collective of the path.
     Returns the mean loss per step (as runner.py:122).  sync_stats=False skips the per-step
     `.item()` host synchronisations of runner.py:108-110 and reads the loss once at the end.
+    presharded=True: the triplets are already this rank's shard (sampling.PairSampler.sample with this rank): they
+    are permuted locally by epoch instead of being split again; gradients are still averaged over the ranks.
     """
     loss_fn = AverageDistortionLoss()
     dev = src_dst_ids.device
     # device_shuffle: the epoch's permutation is drawn on the GPU (not DistributedSampler's CPU order)
-    order = sd.shard_indices(src_dst_ids.shape[0], rank, world_size, epoch=epoch, shuffle=shuffle,
-                             device=dev if device_shuffle else None).to(dev)
+    order = sd.shard_indices(src_dst_ids.shape[0], 0 if presharded else rank, 1 if presharded else world_size, epoch=epoch,
+                             shuffle=shuffle, device=dev if device_shuffle else None).to(dev)
     per_rank = max(batch_size // world_size, 1)
     ok, point, reason = model.check_all_points()        # runner.py:91
     if not ok:
@@ -70,10 +72,15 @@ class FusedEpochRunner:
 
     Restrictions (otherwise use `train_epoch`): float64 CUDA table, grad_accum_steps == 1; the model scale must
     not be trainable (it enters the kernel as a host scalar).  The wsum weights, when the metric has them,
-    are updated as Euclidean parameters with the same clipping coefficient (as geoopt's RSGD does)."""
+    are updated as Euclidean parameters with the same clipping coefficient (as geoopt's RSGD does).
+
+    presharded=True: src_dst_ids / graph_distances are already this rank's shard (sampling.PairSampler.sample with
+    this rank): every epoch permutes all of them locally instead of taking a DistributedSampler shard; gradients
+    are still averaged over the ranks.  run_epoch re-gathers self.ids and self.gdist every epoch, so pairs written
+    into them in place (PairSampler.sample(epoch, out=(runner.ids, runner.gdist))) are trained on at once."""
 
     def __init__(self, model, lr, src_dst_ids, graph_distances, batch_size, max_grad_norm=50.0, world_size=1, rank=0,
-                 use_graph=True, shuffle=True, device_shuffle=False):
+                 use_graph=True, shuffle=True, device_shuffle=False, presharded=False):
         table = model.embeddings.embeds
         if not table.is_cuda or table.dtype != torch.float64:
             raise RuntimeError("FusedEpochRunner needs a CUDA float64 embedding table (there is no CPU path)")
@@ -81,6 +88,8 @@ class FusedEpochRunner:
             raise RuntimeError("FusedEpochRunner: a trainable model scale is not supported, use train_epoch")
         self.model, self.lr, self.max_grad_norm = model, float(lr), float(max_grad_norm)
         self.world, self.rank, self.shuffle, self.device_shuffle = world_size, rank, shuffle, device_shuffle
+        # the split run_epoch takes of self.ids: none when presharded (rank 0 of 1)
+        self.split_rank, self.split_world = (0, 1) if presharded else (rank, world_size)
         self.ids, self.gdist = src_dst_ids, graph_distances
         self.per_rank = max(batch_size // world_size, 1)
         self.dev = table.device
@@ -88,7 +97,7 @@ class FusedEpochRunner:
         self.kind = man.kind
         self.metric = "riem" if self.kind == "spd" else man.metric.name
         self.wsum = getattr(getattr(man, "metric", None), "weights", None) if self.metric == "wsum" else None
-        self.count = -(-src_dst_ids.shape[0] // world_size)     # what shard_indices returns (padded by wrapping)
+        self.count = -(-src_dst_ids.shape[0] // self.split_world)     # what shard_indices returns (padded by wrapping)
         self.idx_buf = torch.empty(self.count, 2, dtype=torch.int64, device=self.dev)
         self.gd_buf = torch.empty(self.count, dtype=torch.float64, device=self.dev)
         self.grad = torch.zeros_like(table.data)
@@ -130,7 +139,7 @@ class FusedEpochRunner:
         ok, point, reason = self.model.check_all_points()        # runner.py:91
         if not ok:
             raise AssertionError(f"Point outside manifold. Reason: {reason}\n{point}")
-        order = sd.shard_indices(self.ids.shape[0], self.rank, self.world, epoch=epoch, shuffle=self.shuffle,
+        order = sd.shard_indices(self.ids.shape[0], self.split_rank, self.split_world, epoch=epoch, shuffle=self.shuffle,
                                  device=self.dev if self.device_shuffle else None).to(self.dev)
         torch.index_select(self.ids, 0, order, out=self.idx_buf)
         torch.index_select(self.gdist, 0, order, out=self.gd_buf)
