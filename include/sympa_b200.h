@@ -38,7 +38,8 @@ extern "C" {
  *    the distance matrix); sympa_hop_distances / _workspace_bytes and sympa_distortion_rows (graph hop
  *    distances by breadth-first search, graph-reconstruction distortion over the same row blocks);
  *    sympa_sample_pairs / _workspace_bytes and SYMPA_STATUS_NO_PAIR (training pairs and their hop distances
- *    sampled by breadth-first search from a list of sources).  Callers
+ *    sampled by breadth-first search from a list of sources); sympa_distortion_rows_full (the distortion terms
+ *    of whole rows, for estimates from sampled nodes).  Callers
  *    that need them look the symbols up; the number stays 4 because nothing that a version-4 caller relies on
  *    changed. */
 #define SYMPA_ABI_VERSION 4
@@ -214,6 +215,15 @@ int sympa_sample_pairs(int64_t num_nodes, const int64_t* adj_ptr, const int64_t*
 int sympa_distortion_rows(int64_t row_begin, int64_t row_count, int64_t num_cols, const double* dist, const int32_t* hops,
                           double scale, double* sum_out, int64_t* count_out, double* max_out, double* min_out,
                           unsigned int* status, void* stream);
+
+/* The same terms over the whole row: for row u = row_begin + r, over every column w != u with hops >= 1 (both
+ * orders of each pair), with the arguments, outputs, NaN and status behaviour of sympa_distortion_rows.  A
+ * sampled node's row is then one unit: sum_out[r] / count_out[r] is the mean distortion of its pairs.  Each row
+ * is summed in one fixed order: bit-identical whatever block, offset or shard it comes in.  Reads 12 bytes per
+ * entry of the row. */
+int sympa_distortion_rows_full(int64_t row_begin, int64_t row_count, int64_t num_cols, const double* dist,
+                               const int32_t* hops, double scale, double* sum_out, int64_t* count_out, double* max_out,
+                               double* min_out, unsigned int* status, void* stream);
 
 /* Backward: replaces autograd through the ~250 torch ops of dist plus the gather backward.
  * grad_dist (num_pairs) is dL/d dist.  Materialised form: grad_z1 / grad_z2 are OVERWRITTEN with

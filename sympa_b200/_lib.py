@@ -51,6 +51,7 @@ EXPORTS = (
     "sympa_hop_distances_workspace_bytes",
     "sympa_hop_distances",
     "sympa_distortion_rows",
+    "sympa_distortion_rows_full",
     "sympa_sample_pairs_workspace_bytes",
     "sympa_sample_pairs",
 )
@@ -128,6 +129,8 @@ def load():
     lib.sympa_hop_distances.argtypes = [L, L, L, P, P, P, P, L, P, P]
     lib.sympa_distortion_rows.restype = I
     lib.sympa_distortion_rows.argtypes = [L, L, L, P, P, D, P, P, P, P, P, P]
+    lib.sympa_distortion_rows_full.restype = I
+    lib.sympa_distortion_rows_full.argtypes = [L, L, L, P, P, D, P, P, P, P, P, P]
     lib.sympa_sample_pairs_workspace_bytes.restype = L
     lib.sympa_sample_pairs_workspace_bytes.argtypes = [L]
     lib.sympa_sample_pairs.restype = I

@@ -1,5 +1,5 @@
 // Graph hop distances and graph-reconstruction distortion of rows of a distance matrix
-// (sympa_hop_distances, sympa_distortion_rows).
+// (sympa_hop_distances, sympa_distortion_rows, sympa_distortion_rows_full).
 //
 //   hop_bfs_kernel         persistent grid, one CTA per source row at a time (rows pulled as tickets from a
 //                          counter at the head of the workspace): level-synchronous breadth-first search whose
@@ -15,10 +15,10 @@
 //                          level loop hop_bfs_levels) into the CTA's own queue and row, then K destinations drawn
 //                          uniformly from the reached set by a binary search over per-word popcount prefixes of
 //                          it; only the K pairs per source reach the output
-//   distortion_rows_kernel one CTA per row: over the columns w > u with a hop distance >= 1, the sum of
-//                          |s d - g| / g, the pair count and the extremes of s d / g; every thread walks a fixed
-//                          residue class of the row's columns and the partial results are combined by a fixed
-//                          tree, so a row's values do not depend on the block it came in
+//   distortion_rows_kernel one CTA per row: over the columns w > u (or, FULL, every column w != u) with a hop
+//                          distance >= 1, the sum of |s d - g| / g, the pair count and the extremes of s d / g;
+//                          every thread walks a fixed residue class of the row's columns and the partial results
+//                          are combined by a fixed tree, so a row's values do not depend on the block it came in
 #pragma once
 
 #include <cooperative_groups.h>
@@ -298,6 +298,10 @@ __global__ void __launch_bounds__(SY_HOP_THREADS, SY_HOP_CTAS_PER_SM) sample_pai
   }
 }
 
+// FULL = false: the columns w > u (sympa_distortion_rows, every pair once); FULL = true: every column w != u
+// (sympa_distortion_rows_full, the whole row of a sampled node).  Thread t walks the columns congruent to its
+// first column modulo SY_DISTORTION_THREADS in both modes.
+template <bool FULL>
 __global__ void __launch_bounds__(SY_DISTORTION_THREADS) distortion_rows_kernel(
     int64_t row_begin, int64_t num_cols, const double* __restrict__ dist, const int* __restrict__ hops, double scale,
     double* __restrict__ sum_out, int64_t* __restrict__ count_out, double* __restrict__ max_out,
@@ -312,10 +316,10 @@ __global__ void __launch_bounds__(SY_DISTORTION_THREADS) distortion_rows_kernel(
   double sum = 0.0, hi = -INFINITY, lo = INFINITY;
   long long cnt = 0;
   int nan = 0;
-  for (int64_t w = u + 1 + threadIdx.x; w < num_cols; w += SY_DISTORTION_THREADS) {
+  for (int64_t w = (FULL ? 0 : u + 1) + threadIdx.x; w < num_cols; w += SY_DISTORTION_THREADS) {
     const int g = __ldcs(hrow + w);
     const double d = __ldcs(drow + w);
-    if (g < 1) continue;
+    if (g < 1 || (FULL && w == u)) continue;
     ++cnt;
     const double sd = scale * d;
     if (isnan(sd)) {

@@ -894,18 +894,36 @@ int sympa_sample_pairs(int64_t num_nodes, const int64_t* adj_ptr, const int64_t*
   return check_launch();
 }
 
-int sympa_distortion_rows(int64_t row_begin, int64_t row_count, int64_t num_cols, const double* dist, const int32_t* hops,
-                          double scale, double* sum_out, int64_t* count_out, double* max_out, double* min_out,
-                          unsigned int* status, void* stream) {
+static int distortion_rows(bool full, int64_t row_begin, int64_t row_count, int64_t num_cols, const double* dist,
+                           const int32_t* hops, double scale, double* sum_out, int64_t* count_out, double* max_out,
+                           double* min_out, unsigned int* status, void* stream) {
   if (row_begin < 0 || row_count < 0 || num_cols < 0 || row_begin + row_count > num_cols || row_count > 0x7FFFFFFFll)
     return SYMPA_ERR_BAD_ARG;
   if (row_count == 0) return SYMPA_OK;
   if (dist == nullptr || hops == nullptr || sum_out == nullptr || count_out == nullptr || max_out == nullptr ||
       min_out == nullptr)
     return SYMPA_ERR_BAD_ARG;
-  distortion_rows_kernel<<<(unsigned)row_count, SY_DISTORTION_THREADS, 0, (cudaStream_t)stream>>>(
-      row_begin, num_cols, dist, hops, scale, sum_out, count_out, max_out, min_out, status);
+  if (full)
+    distortion_rows_kernel<true><<<(unsigned)row_count, SY_DISTORTION_THREADS, 0, (cudaStream_t)stream>>>(
+        row_begin, num_cols, dist, hops, scale, sum_out, count_out, max_out, min_out, status);
+  else
+    distortion_rows_kernel<false><<<(unsigned)row_count, SY_DISTORTION_THREADS, 0, (cudaStream_t)stream>>>(
+        row_begin, num_cols, dist, hops, scale, sum_out, count_out, max_out, min_out, status);
   return check_launch();
+}
+
+int sympa_distortion_rows(int64_t row_begin, int64_t row_count, int64_t num_cols, const double* dist, const int32_t* hops,
+                          double scale, double* sum_out, int64_t* count_out, double* max_out, double* min_out,
+                          unsigned int* status, void* stream) {
+  return distortion_rows(false, row_begin, row_count, num_cols, dist, hops, scale, sum_out, count_out, max_out,
+                         min_out, status, stream);
+}
+
+int sympa_distortion_rows_full(int64_t row_begin, int64_t row_count, int64_t num_cols, const double* dist,
+                               const int32_t* hops, double scale, double* sum_out, int64_t* count_out, double* max_out,
+                               double* min_out, unsigned int* status, void* stream) {
+  return distortion_rows(true, row_begin, row_count, num_cols, dist, hops, scale, sum_out, count_out, max_out,
+                         min_out, status, stream);
 }
 
 int sympa_dist_backward(int kind, int n, int metric, int64_t num_pairs, const double* grad_dist,

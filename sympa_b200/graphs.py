@@ -80,6 +80,25 @@ def adjacency_csr(edges, num_nodes):
     return ptr, idx.contiguous()
 
 
+def relabel_csr(adj, perm):
+    """The CSR adjacency adj = (ptr, idx) with node perm[i] renamed i: new row i is old row perm[i] with every
+    neighbour v renamed inv[v] (inv[perm[i]] = i), entries in their old order.  perm: a permutation of [0, N) as an
+    int64 tensor on adj's device; the work runs there (gathers and one cumulative sum).  Returns (ptr, idx)."""
+    ptr, idx = adj
+    n = ptr.numel() - 1
+    inv = torch.empty_like(perm)
+    inv[perm] = torch.arange(n, dtype=perm.dtype, device=perm.device)
+    start = ptr[:-1][perm]
+    deg = ptr[1:][perm] - start
+    new_ptr = torch.zeros(n + 1, dtype=torch.int64, device=ptr.device)
+    torch.cumsum(deg, 0, out=new_ptr[1:])
+    entries = int(new_ptr[-1])
+    # position in idx of entry j of new row i: start[i] + j = (start[i] - new_ptr[i]) + (new_ptr[i] + j)
+    pos = torch.repeat_interleave(start - new_ptr[:-1], deg, output_size=entries)
+    pos += torch.arange(entries, dtype=torch.int64, device=ptr.device)
+    return new_ptr, inv[idx[pos]]
+
+
 def shortest_path_triplets(adj, block_bytes=1 << 30):
     """(src, dst, distance) triplets of every pair i < j joined by a path in the undirected graph adj = (ptr, idx)
     (adjacency_csr), distance = hop count: the format and order of the generators above, for any graph - what

@@ -25,6 +25,27 @@ i-th hit); with ties it is the "tied nodes rank first" value.  It does not depen
     worst-case distortion = max(s d / g) / min(s d / g) over the same pairs
 
 The reference's evaluate calls model(triplets), so the distances it scores are scaled by s (Model.get_scale()).
+
+Estimates from sampled rows (estimate), for graphs whose N^2 distances and N searches take too long to evaluate
+in full.  The sample is the S nodes with the smallest (h(seed, epoch, 2, node, 0), node) - the SplitMix64 hash of
+sampling.py, tag 2 (tag 1 orders the training sources, tag 0 draws their pairs) - drawn from all N nodes.  Those
+nodes are relabelled 0 .. S-1 in key order (the others follow in id order) and rows [0, S) of the relabelled
+table and graph go through the same pass as evaluate.  A distance comes from the same two table rows wherever
+they sit and hop distances are unique, so a sampled node's AP is bit-identical to its AP in evaluate.  Each
+sampled row u counts every column w != u:
+
+    a_u = sum of delta(u, w) over the w != u connected to u,   c_u = their number   (ops.distortion_rows, full)
+
+    mAP estimate           the mean of AP(u) over the m sampled nodes with neighbours
+    its standard error     sd / sqrt(m) * sqrt(1 - m / M), sd the sample standard deviation (m - 1 in the
+                           denominator) of those AP(u), M the number of nodes with neighbours (from the degrees)
+    average distortion     R = sum a_u / sum c_u, the ratio estimator over the S sampled rows
+    its standard error     SE^2 = (1 - S / N) sum (a_u - R c_u)^2 / ((S - 1) S cbar^2), cbar = sum c_u / S
+    sampled worst case     max(s d / g) / min(s d / g) over the sampled rows' pairs: a LOWER BOUND of the
+                           worst-case distortion (the extremes over a subset of the pairs), with no standard error
+
+At S = N both standard errors are 0 and the estimates equal evaluate's values up to the order of the sums.  A
+standard error that needs two units where there is one (m = 1 < M, or S = 1 < N) is NaN.
 """
 import collections
 import math
@@ -32,11 +53,18 @@ import math
 import torch
 
 from . import distributed as sd
-from . import _lib, ops
+from . import _lib, graphs, ops, sampling
 
 Evaluation = collections.namedtuple("Evaluation", "average_distortion worst_case_distortion mean_ap ap distortion")
 Evaluation.__doc__ = """Result of evaluate(): the two distortion figures and mAP (global when world_size > 1), the (rows,)
 per-node AP of this rank's rows (NaN for a node without neighbours) and their per-node ops.DistortionRows."""
+
+Estimate = collections.namedtuple("Estimate", "mean_ap mean_ap_se average_distortion average_distortion_se "
+                                              "sampled_worst_case_distortion nodes ap distortion")
+Estimate.__doc__ = """Result of estimate(): the estimates of mAP and average distortion with their standard errors, and
+the worst case over the sampled pairs (a lower bound of the exact one), all global when world_size > 1; `nodes` the
+int64 ids of this rank's sampled nodes, `ap` their AP (NaN for a node without neighbours) and `distortion` the
+ops.DistortionRows of their whole rows (every w != u), aligned with `nodes`."""
 
 
 def _adjacency_on(adj, device):
@@ -45,13 +73,16 @@ def _adjacency_on(adj, device):
             torch.as_tensor(idx, dtype=torch.int64).to(device).contiguous())
 
 
-def _row_pass(who, manifold, table, adj, rows, block_bytes, world_size, rank, want_ap, scale):
+def _row_pass(who, manifold, table, adj, rows, block_bytes, world_size, rank, want_ap, scale, perm=None, full=False):
     """The one streaming pass over row blocks of the distance matrix behind every metric here.  Per block:
     dist_matrix, then average_precision (want_ap) and hop_distances + distortion_rows (scale is not None) on that
     same block.  A block holds max(1, block_bytes // (bytes per entry * N)) rows, 8 bytes per entry (distances)
-    plus 4 with distortion (hop distances).  Returns (sums, extremes, ap, distortion): sums = [sum_ap, count_ap]
-    and / or [sum_delta, pairs] and extremes = (max, min) of s d / g, global when world_size > 1 (one SUM
-    all-reduce, one MAX and one MIN), the per-node AP and DistortionRows of this rank's rows."""
+    plus 4 with distortion (hop distances).  perm: the table's rows are taken in this order (table[perm], before
+    the bounded domain's transform, so that one table-sized copy is held); adj must then be relabelled to match.
+    full: the distortion terms of whole rows (ops.distortion_rows(full=True)) instead of the columns w > u.
+    Returns (sums, extremes, ap, distortion): sums = [sum_ap, count_ap] and / or [sum_delta, pairs] and extremes
+    = (max, min) of s d / g, global when world_size > 1 (one SUM all-reduce, one MAX and one MIN), the per-node
+    AP and DistortionRows of this rank's rows."""
     if not isinstance(table, torch.Tensor) or not table.is_cuda:
         raise RuntimeError(f"sympa_b200: {who} needs a CUDA table (there is no CPU path)")
     table = table.detach()
@@ -71,13 +102,14 @@ def _row_pass(who, manifold, table, adj, rows, block_bytes, world_size, rank, wa
     metric = "riem" if kind == "spd" else manifold.metric.name
     wsum = None if kind == "spd" else manifold._wsum(table)
     with torch.cuda.device(dev):
-        src = table
+        src = table if perm is None else table.index_select(0, perm)
         if kind == "bounded":
-            t = ops._require(table, "table")
+            t = ops._require(src, "table")
             ops._check_n(t.shape[-1])
             src = torch.empty_like(t)
             _lib.check(_lib.load().sympa_bounded_rows_to_upper(t.shape[-1], n_nodes, ops._ptr(t), ops._ptr(src),
                                                                ops._ptr(ops.status_word(dev)), ops._stream()))
+            del t
             kind = "upper"
         count_rows = end - begin
         entry_bytes = 12 if want_distortion else 8
@@ -98,7 +130,7 @@ def _row_pass(who, manifold, table, adj, rows, block_bytes, world_size, rank, wa
                 ops.average_precision(d, r0, adj, out=ap[part])
             if want_distortion:
                 h = ops.hop_distances(adj, r0, rc, out=hop_buf[: rc * n_nodes].view(rc, n_nodes))
-                ops.distortion_rows(d, h, r0, scale, out=ops.DistortionRows(*(o[part] for o in dr)))
+                ops.distortion_rows(d, h, r0, scale, out=ops.DistortionRows(*(o[part] for o in dr)), full=full)
         sums = []
         if want_ap:
             valid = ~torch.isnan(ap)
@@ -167,6 +199,98 @@ def evaluate(manifold, table, adj, *, scale=1.0, rows=None, block_bytes=1 << 30,
     return Evaluation(average_distortion=total / pairs if pairs else math.nan,
                       worst_case_distortion=worst_case(hi, lo) if pairs else math.nan,
                       mean_ap=sum_ap / max(count_ap, 1), ap=ap, distortion=dr)
+
+
+def sample_order(num_nodes, num_rows, *, seed=0, epoch=0, device=None):
+    """The permutation of [0, num_nodes) that estimate evaluates under: the num_rows sampled nodes first, in order of
+    (h(seed, epoch, 2, node, 0), node), then the other nodes in id order.  int64 tensor on `device`."""
+    nodes = torch.arange(num_nodes, dtype=torch.int64, device=device)
+    keys = sampling.source_keys(seed, epoch, nodes, tag=2)
+    sample = torch.sort(keys, stable=True).indices[:num_rows]         # ties: by node
+    rest = torch.ones(num_nodes, dtype=torch.bool, device=device)
+    rest[sample] = False
+    return torch.cat((sample, nodes[rest]))
+
+
+def estimate(manifold, table, adj, num_rows, *, scale=1.0, seed=0, epoch=0, block_bytes=1 << 30, world_size=1, rank=0):
+    """mAP and average distortion estimated from num_rows = S sampled rows of the distance matrix of `table` under
+    `manifold` (distances multiplied by `scale`), with their standard errors, as defined in the module docstring:
+    S N distances and S breadth-first searches instead of N^2 and N.  The sample is sample_order(N, S, seed=seed,
+    epoch=epoch); adj = (ptr, idx) as in evaluate.
+
+    The table's rows are gathered in that order (before the bounded domain's transform) and the adjacency is
+    relabelled on the device (graphs.relabel_csr); rows [0, S) then go through evaluate's pass, in blocks of
+    max(1, block_bytes // (12 N)) rows, with the distortion terms of whole rows.  Beyond what evaluate holds (the
+    block, the kernels' workspaces and, for the bounded domain, one transformed table), it holds one permuted
+    table for the other kinds, the relabelled adjacency (8 (N + 1 + E) bytes for E adjacency entries) and, while
+    sampling and relabelling, index arrays of at most 48 N + 24 E bytes.
+    world_size > 1: this rank evaluates its distributed.row_shard part of the S rows; the sums the estimates need
+    are all-reduced over the default process group (one SUM, MAX and MIN, then one SUM of squared deviations), so
+    every figure is global.  Returns an Estimate."""
+    if not isinstance(table, torch.Tensor) or not table.is_cuda:
+        raise RuntimeError("sympa_b200: estimate needs a CUDA table (there is no CPU path)")
+    n_nodes = table.shape[0]
+    num_rows = int(num_rows)
+    if not 1 <= num_rows <= n_nodes:
+        raise ValueError(f"num_rows must lie in [1, {n_nodes}]")
+    seed, epoch = int(seed), int(epoch)
+    if not (0 <= seed < 1 << 64 and 0 <= epoch < 1 << 64):
+        raise ValueError("seed and epoch must lie in [0, 2^64)")
+    dev = table.device
+    scale = float(scale)
+    ptr, idx = _adjacency_on(adj, dev)
+    if ptr.numel() != n_nodes + 1:
+        raise ValueError(f"adj must hold the CSR adjacency of all {n_nodes} nodes")
+    with torch.cuda.device(dev):
+        perm = sample_order(n_nodes, num_rows, seed=seed, epoch=epoch, device=dev)
+        relabelled = graphs.relabel_csr((ptr, idx), perm)
+        with_neighbours = int((ptr[1:] > ptr[:-1]).sum())
+        del ptr, idx
+        (sum_ap, m, sum_a, sum_c), (hi, lo), ap, dr = _row_pass("estimate", manifold, table, relabelled, (0, num_rows),
+                                                                block_bytes, world_size, rank, True, scale, perm=perm,
+                                                                full=True)
+        del relabelled
+        begin, end, _ = sd.row_shard(num_rows, rank, world_size)
+        nodes = perm[begin:end].clone()
+        del perm
+        all_reduce = None
+        if world_size > 1:
+            import torch.distributed as dist
+            all_reduce = dist.all_reduce
+        mean_ap, ap_se, ratio, r_se = _estimates((sum_ap, m, sum_a, sum_c), ap, dr.sum, dr.count, num_rows, n_nodes,
+                                                 with_neighbours, all_reduce)
+    return Estimate(mean_ap=mean_ap, mean_ap_se=ap_se, average_distortion=ratio, average_distortion_se=r_se,
+                    sampled_worst_case_distortion=worst_case(hi, lo) if sum_c else math.nan, nodes=nodes, ap=ap,
+                    distortion=dr)
+
+
+def _estimates(sums, ap, a, c, num_rows, num_nodes, with_neighbours, all_reduce=None):
+    """(mAP, its SE, R, its SE) of the module docstring.  sums = (sum of AP, m, sum of a_u, sum of c_u) over all S
+    sampled rows; ap, a, c: this rank's per-row values (tensors).  The squared deviations from the estimates are
+    summed in a second pass over the rows, and over the ranks by all_reduce (in place, on a tensor) when given."""
+    sum_ap, m, sum_a, sum_c = sums
+    m = int(m)
+    mean_ap = sum_ap / m if m else math.nan
+    ratio = sum_a / sum_c if sum_c else math.nan
+    valid = ~torch.isnan(ap)
+    dev_sq = torch.stack(((ap[valid] - mean_ap).square().sum(), (a - ratio * c.to(torch.float64)).square().sum()))
+    if all_reduce is not None:
+        all_reduce(dev_sq)
+    ss_ap, ss_r = dev_sq.tolist()
+    if m == with_neighbours:
+        ap_se = 0.0
+    elif m < 2:
+        ap_se = math.nan
+    else:
+        ap_se = math.sqrt(ss_ap / (m - 1) / m * (1.0 - m / with_neighbours))
+    if num_rows == num_nodes:
+        r_se = 0.0 if sum_c else math.nan
+    elif num_rows < 2 or not sum_c:
+        r_se = math.nan
+    else:
+        c_bar = sum_c / num_rows
+        r_se = math.sqrt((1.0 - num_rows / num_nodes) * ss_r / ((num_rows - 1) * num_rows * c_bar * c_bar))
+    return mean_ap, ap_se, ratio, r_se
 
 
 def worst_case(max_ratio, min_ratio):

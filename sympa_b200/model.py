@@ -63,6 +63,13 @@ class Model(nn.Module):
         r = evaluate(self.manifold, self.embeddings.embeds, adj, scale=self._eval_scale(), **kw)
         return r.average_distortion, r.mean_ap
 
+    def estimate(self, adj, num_rows, **kw):
+        """mAP and average distortion, with standard errors, estimated from num_rows sampled rows of the distance
+        matrix, distances scaled by get_scale(): the metrics.Estimate of sympa_b200.metrics.estimate (see there for
+        the keywords)."""
+        from .metrics import estimate
+        return estimate(self.manifold, self.embeddings.embeds, adj, num_rows, scale=self._eval_scale(), **kw)
+
     def _eval_scale(self):
         with torch.no_grad():
             return float(self.get_scale().item())

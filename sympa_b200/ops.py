@@ -737,10 +737,11 @@ graph, sum of |s d - g| / g (float64), the number of pairs (int64) and the extre
 -inf / +inf for a row without pairs, NaN for a row with a NaN distance)."""
 
 
-def distortion_rows(dist_block, hop_block, row_begin, scale, out=None):
+def distortion_rows(dist_block, hop_block, row_begin, scale, out=None, full=False):
     """Graph-reconstruction distortion terms of rows [row_begin, row_begin + R) of a distance matrix, from the
     (R, N) float64 block `dist_block` of those rows (dist_matrix) and the (R, N) int32 hop block of the same
-    rows (hop_distances): sympa_distortion_rows.  `scale` multiplies every distance (the model scale).
+    rows (hop_distances): sympa_distortion_rows over the columns w > u, or with full=True
+    sympa_distortion_rows_full over every column w != u.  `scale` multiplies every distance (the model scale).
     Returns a DistortionRows of (R,) tensors; `out` a DistortionRows to write into.  A row's values are
     bit-identical whatever block it comes in.  Parity with the reference's metric code is unpinned (it is not
     available): the definition is the one in include/sympa_b200.h."""
@@ -766,8 +767,9 @@ def distortion_rows(dist_block, hop_block, row_begin, scale, out=None):
     if rows == 0:
         return out
     with torch.cuda.device(dev):
-        _lib.check(lib.sympa_distortion_rows(row_begin, rows, n_cols, _ptr(dist_block), _ptr(hop_block), float(scale),
-                                             *(_ptr(o) for o in out), _ptr(status_word(dev)), _stream()))
+        fn = lib.sympa_distortion_rows_full if full else lib.sympa_distortion_rows
+        _lib.check(fn(row_begin, rows, n_cols, _ptr(dist_block), _ptr(hop_block), float(scale),
+                      *(_ptr(o) for o in out), _ptr(status_word(dev)), _stream()))
     return out
 
 

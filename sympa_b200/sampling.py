@@ -53,10 +53,10 @@ def _mix_tensor(x):
     return x ^ _shr(x, 31)
 
 
-def source_keys(seed, epoch, nodes):
-    """h(seed, epoch, 1, node, 0) of every node of the int64 tensor `nodes`, as int64 tensors whose signed order is
-    the unsigned order of the hash"""
-    head = _i64(_mix(_mix(_mix(seed) ^ epoch) ^ 1))
+def source_keys(seed, epoch, nodes, tag=1):
+    """h(seed, epoch, tag, node, 0) of every node of the int64 tensor `nodes`, as int64 tensors whose signed order is
+    the unsigned order of the hash.  Tag 1 orders the training sources, tag 2 the nodes metrics.estimate samples."""
+    head = _i64(_mix(_mix(_mix(seed) ^ epoch) ^ tag))
     h = _mix_tensor(_mix_tensor(nodes ^ head))
     return h ^ _i64(1 << 63)
 
