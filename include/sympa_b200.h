@@ -39,7 +39,9 @@ extern "C" {
  *    distances by breadth-first search, graph-reconstruction distortion over the same row blocks);
  *    sympa_sample_pairs / _workspace_bytes and SYMPA_STATUS_NO_PAIR (training pairs and their hop distances
  *    sampled by breadth-first search from a list of sources); sympa_distortion_rows_full (the distortion terms
- *    of whole rows, for estimates from sampled nodes).  Callers
+ *    of whole rows, for estimates from sampled nodes); sympa_dist_rows (the distance rows of a list of nodes)
+ *    and sympa_row_topk / _workspace_bytes (the k smallest entries of each row of a distance block, for exact
+ *    k-nearest-neighbour queries).  Callers
  *    that need them look the symbols up; the number stays 4 because nothing that a version-4 caller relies on
  *    changed. */
 #define SYMPA_ABI_VERSION 4
@@ -141,6 +143,34 @@ int sympa_dist_forward(int kind, int n, int metric, int64_t num_pairs,
 int sympa_dist_matrix(int kind, int n, int metric, const double* table, int64_t num_rows,
                       int64_t row_begin, int64_t row_count, const double* wsum_w, double* dist_out,
                       int64_t* idx_workspace, int64_t workspace_pairs, unsigned int* status, void* stream);
+
+/* Distance rows of a LIST of nodes: the (query_count x num_rows) block whose row r is row queries[r] of the matrix
+ * of sympa_dist_matrix, computed the same way (the same chunks of index pairs (queries[r], j) in row-major order,
+ * the same pair kernels, the diagonal pair asked for the next node and then overwritten with 0), so a query row is
+ * bit-identical to the matrix row.  queries: query_count int64 node ids in device memory, repeats allowed.  A query
+ * outside [0, num_rows) cannot be rejected here (the list is not read on the host): its row is NaN and it sets
+ * SYMPA_STATUS_BAD_INDEX; the table is never read outside its rows.  idx_workspace / workspace_pairs as for
+ * sympa_dist_matrix.  Forward only. */
+int sympa_dist_rows(int kind, int n, int metric, const double* table, int64_t num_rows, const int64_t* queries,
+                    int64_t query_count, const double* wsum_w, double* dist_out, int64_t* idx_workspace,
+                    int64_t workspace_pairs, unsigned int* status, void* stream);
+
+/* The k smallest entries of every row of a (row_count x num_cols) float64 block (sympa_dist_rows, sympa_dist_matrix),
+ * without sorting the rows.  The order is total: entries compare by value, -0.0 equal to +0.0, then by column, so
+ * the answer is unique.  Column exclude[r] of row r is left out (exclude: row_count int64, -1 or any value outside
+ * [0, num_cols) leaves nothing out; NULL: nothing is left out for any row).  NaN entries are never selected and set
+ * SYMPA_STATUS_NON_FINITE.  ids_out / dist_out: (row_count x k) int64 columns and float64 values (as stored, -0.0
+ * included), ascending; a row with fewer than k selectable entries is padded with column -1 and value NaN.  Row r
+ * is therefore the stable ascending sort of the row with the excluded column removed, cut to k, each NaN entry
+ * replaced by (-1, NaN).  The output is bit-identical for any block height, row offset, column split or launch
+ * shape.  1 <= k <= 1024: each CTA keeps its k best, k more candidates and one tile of 1024 entries in shared
+ * memory, 16 bytes each, and sorts them there (48 KB at k = 1024, which leaves room for four CTAs per SM).  workspace: device memory, contents irrelevant, of
+ * sympa_row_topk_workspace_bytes(row_count, num_cols, k) bytes (the k best of each of a row's column slices, 16
+ * bytes per candidate; -1 for an argument outside the range).  Reads each entry of the block once, plus k per row. */
+int64_t sympa_row_topk_workspace_bytes(int64_t row_count, int64_t num_cols, int64_t k);
+int sympa_row_topk(int64_t row_count, int64_t num_cols, const double* dist, const int64_t* exclude, int64_t k,
+                   int64_t* ids_out, double* dist_out, void* workspace, int64_t workspace_bytes, unsigned int* status,
+                   void* stream);
 
 /* Graph-reconstruction average precision of rows of a distance matrix (the mAP of the reference's evaluation;
  * its metric code is not available, so parity with it is unpinned - the definition is restated):

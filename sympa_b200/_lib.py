@@ -54,6 +54,9 @@ EXPORTS = (
     "sympa_distortion_rows_full",
     "sympa_sample_pairs_workspace_bytes",
     "sympa_sample_pairs",
+    "sympa_dist_rows",
+    "sympa_row_topk_workspace_bytes",
+    "sympa_row_topk",
 )
 
 _lib = None
@@ -135,6 +138,12 @@ def load():
     lib.sympa_sample_pairs_workspace_bytes.argtypes = [L]
     lib.sympa_sample_pairs.restype = I
     lib.sympa_sample_pairs.argtypes = [L, P, P, L, P, L, ctypes.c_uint64, ctypes.c_uint64, P, P, P, L, P, P]
+    lib.sympa_dist_rows.restype = I
+    lib.sympa_dist_rows.argtypes = [I, I, I, P, L, P, L, P, P, P, L, P, P]
+    lib.sympa_row_topk_workspace_bytes.restype = L
+    lib.sympa_row_topk_workspace_bytes.argtypes = [L, L, L]
+    lib.sympa_row_topk.restype = I
+    lib.sympa_row_topk.argtypes = [L, L, P, P, L, P, P, P, L, P, P]
     _lib = lib
     return lib
 

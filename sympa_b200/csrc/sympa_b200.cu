@@ -9,6 +9,8 @@
 //   hop_bfs_kernel               graph hop distances of a block of source rows (hop_kernels.cuh)
 //   sample_pairs_kernel          training pairs and their hop distances sampled per source (hop_kernels.cuh)
 //   distortion_rows_kernel       graph-reconstruction distortion of distance-matrix rows (hop_kernels.cuh)
+//   query_rows_*_kernel          index pairs and diagonal of the distance rows of a list of nodes (knn_kernels.cuh)
+//   topk_*_kernel                the k smallest entries of each row of a distance block (knn_kernels.cuh)
 #include <cuda_runtime.h>
 #include <stdint.h>
 #include <stdio.h>
@@ -17,6 +19,7 @@
 #include "pair_kernels.cuh"
 #include "ap_kernels.cuh"
 #include "hop_kernels.cuh"
+#include "knn_kernels.cuh"
 
 namespace sympa {
 
@@ -787,6 +790,80 @@ int sympa_dist_matrix(int kind, int n, int metric, const double* table, int64_t 
     return check_launch();
   }
   return SYMPA_OK;
+}
+
+int sympa_dist_rows(int kind, int n, int metric, const double* table, int64_t num_rows, const int64_t* queries,
+                    int64_t query_count, const double* wsum_w, double* dist_out, int64_t* idx_workspace,
+                    int64_t workspace_pairs, unsigned int* status, void* stream) {
+  if (!valid_common(kind, n, metric, 0)) return (n < 1 || n > SYMPA_MAX_N) ? SYMPA_ERR_UNSUPPORTED : SYMPA_ERR_BAD_ARG;
+  if (num_rows <= 0 || query_count < 0) return SYMPA_ERR_BAD_ARG;
+  if (query_count == 0) return SYMPA_OK;
+  if (table == nullptr || queries == nullptr || dist_out == nullptr || idx_workspace == nullptr || workspace_pairs <= 0)
+    return SYMPA_ERR_BAD_ARG;
+  if (metric == SYMPA_METRIC_WSUM && kind != SYMPA_KIND_SPD && wsum_w == nullptr) return SYMPA_ERR_BAD_ARG;
+  cudaStream_t s = (cudaStream_t)stream;
+  const int64_t total = query_count * num_rows;
+  for (int64_t first = 0; first < total; first += workspace_pairs) {
+    const int64_t count = (total - first) < workspace_pairs ? (total - first) : workspace_pairs;
+    query_rows_index_kernel<<<grid_for(count, 256, 8), 256, 0, s>>>(first, count, num_rows, queries,
+                                                                  reinterpret_cast<longlong2*>(idx_workspace));
+    int rc = check_launch();
+    if (rc) return rc;
+    rc = sympa_dist_forward(kind, n, metric, count, nullptr, nullptr, table, num_rows, idx_workspace, wsum_w,
+                            dist_out + first, nullptr, nullptr, nullptr, 0, status, stream);
+    if (rc) return rc;
+  }
+  const int64_t grid = query_count < 65536 ? query_count : 65536;
+  query_rows_fixup_kernel<<<(unsigned)grid, 256, 0, s>>>(query_count, num_rows, queries, dist_out, status);
+  return check_launch();
+}
+
+// CTAs per row of the top-k selection: about 8 CTAs per SM over the whole block, each slice at least 16 columns per
+// thread and 4 k columns (so that a CTA's k survivors are a small part of what it read)
+static int64_t topk_splits(int64_t row_count, int64_t num_cols, int64_t k) {
+  const int64_t want = (int64_t)sm_count() * 8;
+  int64_t splits = (want + row_count - 1) / row_count;
+  int64_t min_slice = (int64_t)SY_KNN_THREADS * 16;
+  if (min_slice < 4 * k) min_slice = 4 * k;
+  const int64_t most = (num_cols + min_slice - 1) / min_slice;
+  if (splits > most) splits = most;
+  if (splits < 1) splits = 1;
+  if (row_count * splits > 0x7FFFFFFFll) splits = 1;
+  return splits;
+}
+
+int64_t sympa_row_topk_workspace_bytes(int64_t row_count, int64_t num_cols, int64_t k) {
+  if (row_count < 0 || row_count > 0x7FFFFFFFll || num_cols < 0 || k < 1 || k > SY_KNN_MAX_K) return -1;
+  if (row_count == 0) return 0;
+  return row_count * topk_splits(row_count, num_cols, k) * k * 16;
+}
+
+int sympa_row_topk(int64_t row_count, int64_t num_cols, const double* dist, const int64_t* exclude, int64_t k,
+                   int64_t* ids_out, double* dist_out, void* workspace, int64_t workspace_bytes, unsigned int* status,
+                   void* stream) {
+  const int64_t need = sympa_row_topk_workspace_bytes(row_count, num_cols, k);
+  if (need < 0) return SYMPA_ERR_BAD_ARG;
+  if (row_count == 0) return SYMPA_OK;
+  if ((dist == nullptr && num_cols > 0) || ids_out == nullptr || dist_out == nullptr || workspace == nullptr ||
+      workspace_bytes < need)
+    return SYMPA_ERR_BAD_ARG;
+  cudaStream_t s = (cudaStream_t)stream;
+  const int64_t splits = topk_splits(row_count, num_cols, k);
+  const int buf = knn_buffer_entries(k);
+  const size_t smem = (size_t)buf * 16;
+  static_assert(2 * SY_KNN_MAX_K + SY_KNN_TILE <= 3072, "the largest buffer must stay within 48 KB");
+  // above 48 KB of shared memory per CTA (with the static part) a kernel has to opt in
+  if (cudaFuncSetAttribute(topk_select_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem) != cudaSuccess ||
+      cudaFuncSetAttribute(topk_merge_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem) != cudaSuccess)
+    return check_launch();
+  longlong2* cand = static_cast<longlong2*>(workspace);
+  topk_select_kernel<<<(unsigned)(row_count * splits), SY_KNN_THREADS, smem, s>>>(num_cols, (int)splits, (int)k, buf,
+                                                                                 dist, exclude, cand, status);
+  int rc = check_launch();
+  if (rc) return rc;
+  topk_merge_kernel<<<(unsigned)row_count, SY_KNN_THREADS, smem, s>>>(num_cols, (int)splits, (int)k, buf, dist, cand,
+                                                                      ids_out, dist_out);
+  return check_launch();
 }
 
 int64_t sympa_average_precision_workspace_bytes(int64_t row_count, int64_t adj_entries) {

@@ -46,6 +46,10 @@ sampled row u counts every column w != u:
 
 At S = N both standard errors are 0 and the estimates equal evaluate's values up to the order of the sums.  A
 standard error that needs two units where there is one (m = 1 < M, or S = 1 < N) is NaN.
+
+Exact k-nearest-neighbour queries (nearest): the distance rows of the query nodes (sympa_dist_rows, bit-identical
+to the rows of sympa_dist_matrix) are computed in blocks and each block is reduced on the device to the k smallest
+entries of every row (sympa_row_topk), in the total order (distance, node id).
 """
 import collections
 import math
@@ -66,11 +70,40 @@ the worst case over the sampled pairs (a lower bound of the exact one), all glob
 int64 ids of this rank's sampled nodes, `ap` their AP (NaN for a node without neighbours) and `distortion` the
 ops.DistortionRows of their whole rows (every w != u), aligned with `nodes`."""
 
+Neighbours = collections.namedtuple("Neighbours", "ids distances")
+Neighbours.__doc__ = """Result of nearest(): (Q, k) int64 node ids and float64 scaled distances, row i the k nearest nodes of
+queries[i] in ascending order of distance, then of id; (-1, NaN) past the selectable nodes of a row."""
+
 
 def _adjacency_on(adj, device):
     ptr, idx = adj
     return (torch.as_tensor(ptr, dtype=torch.int64).to(device).contiguous(),
             torch.as_tensor(idx, dtype=torch.int64).to(device).contiguous())
+
+
+def _cuda_table(who, table):
+    if not isinstance(table, torch.Tensor) or not table.is_cuda:
+        raise RuntimeError(f"sympa_b200: {who} needs a CUDA table (there is no CPU path)")
+    return table.detach()
+
+
+def _distance_source(manifold, table, perm=None):
+    """(src, kind, metric, wsum) for the distance kernels, on the current device: the table (its rows in the order
+    perm when given) or, for the bounded domain, its inverse Cayley transform (sympa_bounded_rows_to_upper, once per
+    table) with kind "upper"; spd takes the riem kernels and no weights."""
+    kind = manifold.kind
+    metric = "riem" if kind == "spd" else manifold.metric.name
+    wsum = None if kind == "spd" else manifold._wsum(table)
+    src = table if perm is None else table.index_select(0, perm)
+    if kind == "bounded":
+        t = ops._require(src, "table")
+        ops._check_n(t.shape[-1])
+        src = torch.empty_like(t)
+        _lib.check(_lib.load().sympa_bounded_rows_to_upper(t.shape[-1], t.shape[0], ops._ptr(t), ops._ptr(src),
+                                                           ops._ptr(ops.status_word(t.device)), ops._stream()))
+        del t
+        kind = "upper"
+    return src, kind, metric, wsum
 
 
 def _row_pass(who, manifold, table, adj, rows, block_bytes, world_size, rank, want_ap, scale, perm=None, full=False):
@@ -83,9 +116,7 @@ def _row_pass(who, manifold, table, adj, rows, block_bytes, world_size, rank, wa
     Returns (sums, extremes, ap, distortion): sums = [sum_ap, count_ap] and / or [sum_delta, pairs] and extremes
     = (max, min) of s d / g, global when world_size > 1 (one SUM all-reduce, one MAX and one MIN), the per-node
     AP and DistortionRows of this rank's rows."""
-    if not isinstance(table, torch.Tensor) or not table.is_cuda:
-        raise RuntimeError(f"sympa_b200: {who} needs a CUDA table (there is no CPU path)")
-    table = table.detach()
+    table = _cuda_table(who, table)
     dev = table.device
     n_nodes = table.shape[0]
     begin, end = (0, n_nodes) if rows is None else (int(rows[0]), int(rows[1]))
@@ -98,19 +129,8 @@ def _row_pass(who, manifold, table, adj, rows, block_bytes, world_size, rank, wa
     want_distortion = scale is not None
     if want_distortion:
         scale = float(scale)
-    kind = manifold.kind
-    metric = "riem" if kind == "spd" else manifold.metric.name
-    wsum = None if kind == "spd" else manifold._wsum(table)
     with torch.cuda.device(dev):
-        src = table if perm is None else table.index_select(0, perm)
-        if kind == "bounded":
-            t = ops._require(src, "table")
-            ops._check_n(t.shape[-1])
-            src = torch.empty_like(t)
-            _lib.check(_lib.load().sympa_bounded_rows_to_upper(t.shape[-1], n_nodes, ops._ptr(t), ops._ptr(src),
-                                                               ops._ptr(ops.status_word(dev)), ops._stream()))
-            del t
-            kind = "upper"
+        src, kind, metric, wsum = _distance_source(manifold, table, perm)
         count_rows = end - begin
         entry_bytes = 12 if want_distortion else 8
         block = max(1, min(block_bytes // (entry_bytes * max(n_nodes, 1)), max(count_rows, 1)))
@@ -199,6 +219,58 @@ def evaluate(manifold, table, adj, *, scale=1.0, rows=None, block_bytes=1 << 30,
     return Evaluation(average_distortion=total / pairs if pairs else math.nan,
                       worst_case_distortion=worst_case(hi, lo) if pairs else math.nan,
                       mean_ap=sum_ap / max(count_ap, 1), ap=ap, distortion=dr)
+
+
+def nearest(manifold, table, queries, k, *, scale=1.0, exclude_self=True, block_bytes=1 << 30, world_size=1, rank=0):
+    """The k nearest nodes of every node in `queries` under `manifold`, exactly: a Neighbours of (Q, k) ids (int64)
+    and distances (float64, multiplied by `scale`) on the table's device, nearest first.  Row i is the stable
+    ascending sort of row queries[i] of the distance matrix (ties by node id, -0.0 equal to +0.0), without the query
+    node itself when exclude_self, cut to k; NaN distances are never selected (the status check raises) and a row
+    with fewer than k selectable nodes is padded with (-1, NaN).
+
+    queries: 1-D int64 tensor of node ids in [0, N), repeats allowed, possibly empty; 1 <= k <= min(1024, N - 1)
+    with exclude_self (N without).  Both are checked before any launch.  The queries go through in blocks of
+    max(1, block_bytes // (8 N)) rows, one reused block buffer: their distance rows (ops.dist_rows, bit-identical to
+    the rows of dist_matrix; the bounded domain on its inverse Cayley transform, once per table, as in evaluate),
+    then the k smallest of each row (ops.row_topk).  Beyond the block it holds the (Q, k) outputs and the two
+    kernels' workspaces.  world_size > 1: this rank answers its distributed.row_shard part of the queries (no
+    collective).  The status word is checked once, at the end."""
+    if not isinstance(table, torch.Tensor):
+        raise TypeError("table must be a tensor")
+    if not isinstance(queries, torch.Tensor) or queries.dtype != torch.int64:
+        raise TypeError("queries must be an int64 tensor")
+    if queries.dim() != 1:
+        raise ValueError("queries must be 1-D")
+    n_nodes = table.shape[0]
+    k = int(k)
+    top = min(ops.TOPK_MAX_K, n_nodes - bool(exclude_self))
+    if not 1 <= k <= top:
+        raise ValueError(f"k must lie in [1, {top}]" if top >= 1 else f"a table of {n_nodes} nodes has no neighbour to return")
+    if queries.numel() and (int(queries.min()) < 0 or int(queries.max()) >= n_nodes):
+        raise ValueError(f"queries must lie in [0, {n_nodes})")
+    table = _cuda_table("nearest", table)
+    dev = table.device
+    if world_size > 1:
+        lo, hi, _ = sd.row_shard(queries.numel(), rank, world_size)
+        queries = queries[lo:hi]
+    with torch.cuda.device(dev):
+        queries = queries.to(dev).contiguous()
+        count = queries.numel()
+        ids = torch.empty(count, k, dtype=torch.int64, device=dev)
+        dist = torch.empty(count, k, dtype=torch.float64, device=dev)
+        if count:
+            src, kind, metric, wsum = _distance_source(manifold, table)
+            block = max(1, min(block_bytes // (8 * n_nodes), count))
+            buf = torch.empty(block * n_nodes, dtype=torch.float64, device=dev)
+            for q0 in range(0, count, block):
+                qc = min(block, count - q0)
+                q = queries[q0:q0 + qc]
+                d = ops.dist_rows(kind, metric, src, q, wsum, out=buf[: qc * n_nodes].view(qc, n_nodes))
+                ops.row_topk(d, k, exclude=q if exclude_self else None, out=(ids[q0:q0 + qc], dist[q0:q0 + qc]))
+            del buf, src
+            dist.mul_(float(scale))
+        ops.check_status(dev)
+    return Neighbours(ids, dist)
 
 
 def sample_order(num_nodes, num_rows, *, seed=0, epoch=0, device=None):

@@ -70,6 +70,12 @@ class Model(nn.Module):
         from .metrics import estimate
         return estimate(self.manifold, self.embeddings.embeds, adj, num_rows, scale=self._eval_scale(), **kw)
 
+    def nearest(self, queries, k, **kw):
+        """The k nearest nodes of every node in `queries` (1-D int64 ids), distances scaled by get_scale(): the
+        metrics.Neighbours of sympa_b200.metrics.nearest (see there for the keywords)."""
+        from .metrics import nearest
+        return nearest(self.manifold, self.embeddings.embeds, queries, k, scale=self._eval_scale(), **kw)
+
     def _eval_scale(self):
         with torch.no_grad():
             return float(self.get_scale().item())

@@ -573,13 +573,104 @@ def dist_matrix(kind, metric, table, row_begin=0, row_count=None, wsum_w=None, c
         if row_count == 0 or rows == 0:
             return out
         chunk = max(1, min(chunk_pairs, row_count * rows))
-        key = (dev.type, dev.index if dev.index is not None else torch.cuda.current_device())
-        ws = _idx_workspace.get(key)
-        if ws is None or ws.numel() < 2 * chunk:
-            ws = torch.empty(2 * chunk, dtype=torch.int64, device=dev)
-            _idx_workspace[key] = ws
+        ws = _idx_workspace_for(dev, chunk)
         _lib.check(lib.sympa_dist_matrix(_lib.KIND[kind], n, _lib.METRIC[metric], _ptr(table), rows, row_begin, row_count,
                                          _ptr(wsum_w), _ptr(out), _ptr(ws), chunk, _ptr(status_word(dev)), _stream()))
+    return out
+
+
+def _idx_workspace_for(dev, chunk):
+    """the per-device index workspace of dist_matrix and dist_rows, grown to 2 * chunk int64 on demand"""
+    key = (dev.type, dev.index if dev.index is not None else torch.cuda.current_device())
+    ws = _idx_workspace.get(key)
+    if ws is None or ws.numel() < 2 * chunk:
+        ws = torch.empty(2 * chunk, dtype=torch.int64, device=dev)
+        _idx_workspace[key] = ws
+    return ws
+
+
+def dist_rows(kind, metric, table, queries, wsum_w=None, out=None, chunk_pairs=1 << 24):
+    """Rows queries[0], queries[1], ... of the all-pairs distance matrix of `table` (forward only): sympa_dist_rows,
+    each row bit-identical to the same row of dist_matrix.  queries: 1-D int64 node ids on the table's device, in
+    [0, N) (checked here, one host synchronisation), repeats allowed.  Returns the (Q, N) float64 block; `out` a
+    contiguous (Q, N) float64 tensor to write into.  The index workspace is dist_matrix's, shared per device."""
+    lib = _lib.load()
+    table = _require(table, "table").detach()
+    queries = _require(queries, "queries", torch.int64)
+    n = table.shape[-1]
+    _check_n(n)
+    rows = table.shape[0]
+    dev = table.device
+    if queries.dim() != 1 or queries.device != dev:
+        raise ValueError(f"queries must be a 1-D tensor on {dev}")
+    q = queries.numel()
+    if q and (rows == 0 or int(queries.min()) < 0 or int(queries.max()) >= rows):
+        raise ValueError(f"queries must lie in [0, {rows})")
+    if metric == "wsum" and kind != "spd":
+        wsum_w = _require(wsum_w, "wsum_w").reshape(-1)
+    else:
+        wsum_w = None
+    with torch.cuda.device(dev):
+        if out is None:
+            out = torch.empty(q, rows, dtype=torch.float64, device=dev)
+        elif out.dtype != torch.float64 or out.device != dev or tuple(out.shape) != (q, rows) or not out.is_contiguous():
+            raise ValueError(f"out must be a contiguous float64 ({q}, {rows}) tensor on {dev}")
+        if q == 0:
+            return out
+        chunk = max(1, min(chunk_pairs, q * rows))
+        ws = _idx_workspace_for(dev, chunk)
+        _lib.check(lib.sympa_dist_rows(_lib.KIND[kind], n, _lib.METRIC[metric], _ptr(table), rows, _ptr(queries), q,
+                                       _ptr(wsum_w), _ptr(out), _ptr(ws), chunk, _ptr(status_word(dev)), _stream()))
+    return out
+
+
+_topk_workspace = {}
+TOPK_MAX_K = 1024
+
+
+def row_topk(dist_block, k, exclude=None, out=None):
+    """The k smallest entries of every row of the (R, M) float64 block `dist_block`: sympa_row_topk.  Entries
+    compare by value (-0.0 equal to +0.0), then by column; column exclude[r] (1-D int64 on the block's device, -1
+    for none) is left out of row r; NaN entries are never selected (they set the non-finite status bit).  Returns
+    (ids (R, k) int64, values (R, k) float64), ascending, a row with fewer than k selectable entries padded with
+    (-1, NaN): row r equals torch.sort(row, stable=True) with the excluded column removed, cut to k, NaN entries
+    replaced by (-1, NaN).  1 <= k <= 1024.  `out` = (ids, values) to write into.  The workspace (16 bytes per
+    candidate of a column slice) is kept per device and reused."""
+    lib = _lib.load()
+    dist_block = _require(dist_block, "dist_block")
+    if dist_block.dim() != 2:
+        raise ValueError("dist_block must be (rows, columns)")
+    rows, cols = dist_block.shape
+    dev = dist_block.device
+    k = int(k)
+    if not 1 <= k <= TOPK_MAX_K:
+        raise ValueError(f"k must lie in [1, {TOPK_MAX_K}]")
+    if exclude is not None:
+        exclude = _require(exclude, "exclude", torch.int64)
+        if exclude.device != dev or tuple(exclude.shape) != (rows,):
+            raise ValueError(f"exclude must be a ({rows},) tensor on {dev}")
+    if out is None:
+        out = (torch.empty(rows, k, dtype=torch.int64, device=dev), torch.empty(rows, k, dtype=torch.float64, device=dev))
+    else:
+        ids, vals = out
+        if (ids.dtype != torch.int64 or ids.device != dev or tuple(ids.shape) != (rows, k) or not ids.is_contiguous()
+                or vals.dtype != torch.float64 or vals.device != dev or tuple(vals.shape) != (rows, k)
+                or not vals.is_contiguous()):
+            raise ValueError(f"out must be contiguous int64 and float64 ({rows}, {k}) tensors on {dev}")
+        out = (ids, vals)
+    if rows == 0:
+        return out
+    with torch.cuda.device(dev):
+        nbytes = lib.sympa_row_topk_workspace_bytes(rows, cols, k)
+        if nbytes < 0:
+            raise ValueError(f"at most 2^31 - 1 rows per call, got {rows}")
+        key = (dev.type, dev.index if dev.index is not None else torch.cuda.current_device())
+        ws = _topk_workspace.get(key)
+        if ws is None or ws.numel() * 8 < nbytes:
+            ws = torch.empty((nbytes + 7) // 8, dtype=torch.float64, device=dev)
+            _topk_workspace[key] = ws
+        _lib.check(lib.sympa_row_topk(rows, cols, _ptr(dist_block), _ptr(exclude), k, _ptr(out[0]), _ptr(out[1]), _ptr(ws),
+                                      ws.numel() * 8, _ptr(status_word(dev)), _stream()))
     return out
 
 
