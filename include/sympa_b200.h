@@ -41,8 +41,8 @@ extern "C" {
  *    sampled by breadth-first search from a list of sources); sympa_distortion_rows_full (the distortion terms
  *    of whole rows, for estimates from sampled nodes); sympa_dist_rows (the distance rows of a list of nodes)
  *    and sympa_row_topk / _workspace_bytes (the k smallest entries of each row of a distance block, for exact
- *    k-nearest-neighbour queries).  Callers
- *    that need them look the symbols up; the number stays 4 because nothing that a version-4 caller relies on
+ *    k-nearest-neighbour queries); sympa_target_ranks / _workspace_bytes (filtered ranks of held-out targets among
+ *    all nodes, for link-prediction evaluation).  Callers that need them look the symbols up; the number stays 4 because nothing that a version-4 caller relies on
  *    changed. */
 #define SYMPA_ABI_VERSION 4
 
@@ -171,6 +171,34 @@ int64_t sympa_row_topk_workspace_bytes(int64_t row_count, int64_t num_cols, int6
 int sympa_row_topk(int64_t row_count, int64_t num_cols, const double* dist, const int64_t* exclude, int64_t k,
                    int64_t* ids_out, double* dist_out, void* workspace, int64_t workspace_bytes, unsigned int* status,
                    void* stream);
+
+/* Filtered ranks of held-out targets, for link-prediction evaluation (the definition is the project's own: the
+ * reference has no link-prediction code).  With d(u, w) row u of the matrix of sympa_dist_matrix, for a directed
+ * query pair (u, v), u != v, and the filter row F(u) (the known neighbours of u):
+ *   C(u, v) = {w in [0, num_cols) : w != u, w != v, w not in F(u)}                        competitors
+ *   lt(u, v) = |{w in C : d(u,w) < d(u,v)}|,   le(u, v) = |{w in C : d(u,w) <= d(u,v)}|
+ *   optimistic rank = 1 + lt,   pessimistic rank = 1 + le,   rank = 1 + (lt + le) / 2     (ties split)
+ * -0.0 equals +0.0 and +-inf compare as usual.  A NaN anywhere in row u (w != u) makes every pair of the row
+ * undefined: lt = le = -1, and it sets SYMPA_STATUS_NON_FINITE.  All counts are integers, so a pair's result is
+ * exact and bit-identical for any block height, offset or launch shape.
+ * dist: the (row_count x num_cols) float64 block whose row r is row queries[r] of the matrix (sympa_dist_rows).
+ * target_ptr (row_count + 1) / target_idx: the targets of block row r are target_idx[target_ptr[r] ..
+ * target_ptr[r + 1]), repeats allowed; lt_out[i] / le_out[i] (int64) are written for every entry i in
+ * [target_ptr[0], target_ptr[row_count]), the same indexing as target_idx.  A target outside [0, num_cols) gets -1
+ * and sets SYMPA_STATUS_BAD_INDEX; so does every target of a row whose query lies outside [0, num_cols).  A row
+ * without targets is not read.
+ * filter_ptr (num_cols + 1) / filter_idx: CSR filter adjacency of all nodes (valid pointers), each row sorted and free
+ * of duplicates (graphs.adjacency_csr); an empty adjacency is the "raw" setting.  Entries equal to the row's node
+ * are ignored, entries outside [0, num_cols) are skipped and set SYMPA_STATUS_BAD_INDEX.
+ * workspace: device memory, contents irrelevant, of sympa_target_ranks_workspace_bytes(row_count, target_entries)
+ * bytes where target_entries >= target_ptr[row_count] - target_ptr[0]; rows whose targets do not fit get -1 and set
+ * SYMPA_STATUS_BAD_INDEX.  Reads each entry of the block once, plus the targets' and the filter rows' entries; rows
+ * of up to 2048 targets count in shared memory, longer ones in the workspace. */
+int64_t sympa_target_ranks_workspace_bytes(int64_t row_count, int64_t target_entries);
+int sympa_target_ranks(int64_t row_count, int64_t num_cols, const double* dist, const int64_t* queries,
+                       const int64_t* target_ptr, const int64_t* target_idx, const int64_t* filter_ptr,
+                       const int64_t* filter_idx, int64_t* lt_out, int64_t* le_out, void* workspace,
+                       int64_t workspace_bytes, unsigned int* status, void* stream);
 
 /* Graph-reconstruction average precision of rows of a distance matrix (the mAP of the reference's evaluation;
  * its metric code is not available, so parity with it is unpinned - the definition is restated):

@@ -57,6 +57,8 @@ EXPORTS = (
     "sympa_dist_rows",
     "sympa_row_topk_workspace_bytes",
     "sympa_row_topk",
+    "sympa_target_ranks_workspace_bytes",
+    "sympa_target_ranks",
 )
 
 _lib = None
@@ -144,6 +146,10 @@ def load():
     lib.sympa_row_topk_workspace_bytes.argtypes = [L, L, L]
     lib.sympa_row_topk.restype = I
     lib.sympa_row_topk.argtypes = [L, L, P, P, L, P, P, P, L, P, P]
+    lib.sympa_target_ranks_workspace_bytes.restype = L
+    lib.sympa_target_ranks_workspace_bytes.argtypes = [L, L]
+    lib.sympa_target_ranks.restype = I
+    lib.sympa_target_ranks.argtypes = [L, L, P, P, P, P, P, P, P, P, P, L, P, P]
     _lib = lib
     return lib
 

@@ -20,6 +20,7 @@
 #include "ap_kernels.cuh"
 #include "hop_kernels.cuh"
 #include "knn_kernels.cuh"
+#include "rank_kernels.cuh"
 
 namespace sympa {
 
@@ -902,6 +903,51 @@ int sympa_average_precision(int64_t row_begin, int64_t row_count, int64_t num_co
   if (rc) return rc;
   ap_finish_kernel<<<(unsigned)((row_count + SY_AP_THREADS - 1) / SY_AP_THREADS), SY_AP_THREADS, 0, s>>>(
       row_begin, row_count, adj_ptr, meta, sorted, counts, ap_out);
+  return check_launch();
+}
+
+int64_t sympa_target_ranks_workspace_bytes(int64_t row_count, int64_t target_entries) {
+  if (row_count < 0 || target_entries < 0) return -1;
+  return (row_count + 3 * target_entries) * (int64_t)sizeof(double);
+}
+
+int sympa_target_ranks(int64_t row_count, int64_t num_cols, const double* dist, const int64_t* queries,
+                       const int64_t* target_ptr, const int64_t* target_idx, const int64_t* filter_ptr,
+                       const int64_t* filter_idx, int64_t* lt_out, int64_t* le_out, void* workspace,
+                       int64_t workspace_bytes, unsigned int* status, void* stream) {
+  if (row_count < 0 || num_cols <= 0 || row_count > 0x7FFFFFFFll) return SYMPA_ERR_BAD_ARG;
+  if (row_count == 0) return SYMPA_OK;
+  if (dist == nullptr || queries == nullptr || target_ptr == nullptr || target_idx == nullptr || filter_ptr == nullptr ||
+      filter_idx == nullptr || lt_out == nullptr || le_out == nullptr || workspace == nullptr)
+    return SYMPA_ERR_BAD_ARG;
+  if (workspace_bytes < sympa_target_ranks_workspace_bytes(row_count, 0)) return SYMPA_ERR_BAD_ARG;
+  const int64_t cap = (workspace_bytes / (int64_t)sizeof(double) - row_count) / 3;
+  cudaStream_t s = (cudaStream_t)stream;
+  unsigned long long* flags = static_cast<unsigned long long*>(workspace);
+  double* sorted = reinterpret_cast<double*>(flags + row_count);
+  unsigned long long* le_bins = reinterpret_cast<unsigned long long*>(sorted + cap);
+  unsigned long long* eq_bins = le_bins + cap;
+  rank_prepare_kernel<<<(unsigned)row_count, SY_RANK_THREADS, 0, s>>>(num_cols, dist, queries, target_ptr, target_idx, cap,
+                                                                     flags, sorted, le_bins, eq_bins, status);
+  int rc = check_launch();
+  if (rc) return rc;
+  // split each row over several CTAs until the grid is ~8 CTAs per SM, each CTA keeping >= 16 columns per thread
+  // and (for the shared 32-bit bins) fewer than 2^32 columns
+  const int64_t want = (int64_t)sm_count() * 8;
+  int64_t splits = (want + row_count - 1) / row_count;
+  const int64_t most = (num_cols + SY_RANK_THREADS * 16 - 1) / (SY_RANK_THREADS * 16);
+  if (splits > most) splits = most;
+  const int64_t least = (num_cols >> 32) + 1;
+  if (splits < least) splits = least;
+  if (row_count * splits > 0x7FFFFFFFll) return SYMPA_ERR_BAD_ARG;
+  rank_count_kernel<<<(unsigned)(row_count * splits), SY_RANK_THREADS, 0, s>>>(num_cols, (int)splits, dist, queries,
+                                                                               target_ptr, flags, sorted, le_bins, eq_bins,
+                                                                               status);
+  rc = check_launch();
+  if (rc) return rc;
+  rank_finish_kernel<<<(unsigned)row_count, SY_RANK_THREADS, 0, s>>>(num_cols, dist, queries, target_ptr, target_idx,
+                                                                    filter_ptr, filter_idx, flags, sorted, le_bins,
+                                                                    eq_bins, lt_out, le_out, status);
   return check_launch();
 }
 

@@ -80,6 +80,39 @@ def adjacency_csr(edges, num_nodes):
     return ptr, idx.contiguous()
 
 
+def split_edges(edges, num_nodes, test_fraction, *, seed=0):
+    """(train_edges, test_edges): a deterministic split of the undirected graph with the (E, 2) int64 node pairs
+    `edges` over [0, num_nodes), for link-prediction evaluation.  The edges are canonicalised to (min, max), self
+    loops and duplicates removed; of the E' left, the round(test_fraction E') with the smallest
+    (h(seed, 0, 3, u, v), u, v) are held out, h the SplitMix64 hash of sampling.py (tag 3).  Both outputs are (., 2)
+    int64, sorted by (u, v), on the device of `edges`, and identical on CPU and CUDA tensors.  A node can lose all of
+    its training edges; metrics.link_prediction still ranks its held-out targets.  Typical use: the training graph
+    adjacency_csr(train_edges, n) for sampling.PairSampler, the test pairs torch.cat((test, test.flip(1))) and the
+    filter adjacency_csr(edges, n)."""
+    from . import sampling
+
+    edges = torch.as_tensor(edges)
+    if edges.dtype != torch.int64 or edges.dim() != 2 or edges.shape[1] != 2:
+        raise ValueError("edges must be an (E, 2) int64 tensor")
+    if edges.numel() and (int(edges.min()) < 0 or int(edges.max()) >= num_nodes):
+        raise ValueError(f"edge endpoints must lie in [0, {num_nodes})")
+    test_fraction = float(test_fraction)
+    if not 0.0 <= test_fraction <= 1.0:
+        raise ValueError("test_fraction must lie in [0, 1]")
+    seed = int(seed)
+    if not 0 <= seed < 1 << 64:
+        raise ValueError("seed must lie in [0, 2^64)")
+    lo, hi = torch.minimum(edges[:, 0], edges[:, 1]), torch.maximum(edges[:, 0], edges[:, 1])
+    key = torch.unique((lo * num_nodes + hi)[lo != hi])               # sorted: by u, then by v
+    u, v = key // num_nodes, key % num_nodes
+    held = round(test_fraction * key.numel())
+    order = torch.sort(sampling.source_keys(seed, 0, u, tag=3, second=v), stable=True).indices   # ties: by (u, v)
+    test = torch.zeros(key.numel(), dtype=torch.bool, device=edges.device)
+    test[order[:held]] = True
+    both = torch.stack((u, v), 1)
+    return both[~test].contiguous(), both[test].contiguous()
+
+
 def relabel_csr(adj, perm):
     """The CSR adjacency adj = (ptr, idx) with node perm[i] renamed i: new row i is old row perm[i] with every
     neighbour v renamed inv[v] (inv[perm[i]] = i), entries in their old order.  perm: a permutation of [0, N) as an

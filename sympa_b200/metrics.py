@@ -50,6 +50,24 @@ standard error that needs two units where there is one (m = 1 < M, or S = 1 < N)
 Exact k-nearest-neighbour queries (nearest): the distance rows of the query nodes (sympa_dist_rows, bit-identical
 to the rows of sympa_dist_matrix) are computed in blocks and each block is reduced on the device to the k smallest
 entries of every row (sympa_row_topk), in the total order (distance, node id).
+
+Link prediction (link_prediction) - the definition is the project's own (the reference has no link-prediction code,
+so parity is unpinned).  The inputs are directed query pairs (u, v), u != v, v the held-out target of u, and a filter
+adjacency F (graphs.adjacency_csr; F(u) the known neighbours of u, usually the whole graph, training and held-out
+edges; an adjacency without edges gives the "raw" setting).  With d row u of the distance matrix:
+
+    C(u, v)     = {w in [0, N) : w != u, w != v, w not in F(u)}                     competitors
+    lt(u, v)    = |{w in C : d(u,w) <  d(u,v)}|
+    le(u, v)    = |{w in C : d(u,w) <= d(u,v)}|
+    optimistic  = 1 + lt,   pessimistic = 1 + le,   rank = 1 + (lt + le) / 2          (ties split)
+    MRR         = mean over the pairs of 1 / rank
+    Hits@k      = mean over the pairs of [rank <= k]
+
+-0.0 equals +0.0 and +-inf compare as usual.  A NaN anywhere in row u (w != u) makes the ranks of every pair of u
+NaN, and the status check raises, as for AP.  Ranks do not depend on the model scale.  Splitting ties gives a
+collapsed embedding, every distance equal, a middle rank rather than rank 1.  All counts are integers, so a pair's
+ranks are exact and do not depend on the block, the rank shard or the launch shape.  Pairs are directed: to rank both
+endpoints of undirected held-out edges e, pass torch.cat((e, e.flip(1))).
 """
 import collections
 import math
@@ -271,6 +289,92 @@ def nearest(manifold, table, queries, k, *, scale=1.0, exclude_self=True, block_
             dist.mul_(float(scale))
         ops.check_status(dev)
     return Neighbours(ids, dist)
+
+
+LinkPrediction = collections.namedtuple("LinkPrediction", "mrr hits count pairs rank optimistic pessimistic")
+LinkPrediction.__doc__ = """Result of link_prediction(): MRR, `hits` = {k: Hits@k} and the number of pairs, global when
+world_size > 1; `pairs` the int64 positions in the input of this rank's pairs, ascending, and `rank`, `optimistic`,
+`pessimistic` their float64 ranks (module docstring), aligned with `pairs`."""
+
+
+def link_prediction(manifold, table, pairs, filter_adj, *, ks=(1, 3, 10), block_bytes=1 << 30, world_size=1, rank=0):
+    """Filtered link-prediction ranks of the directed query pairs `pairs` ((E, 2) int64 (u, v), v the held-out target
+    of u, ids in [0, N), u != v) among all N nodes under `manifold`, with MRR and Hits@k for every k in `ks`, as
+    defined in the module docstring.  filter_adj = (ptr, idx): the CSR adjacency (graphs.adjacency_csr) of the known
+    edges left out of the competitors, moved to the table's device.  pairs, ks and the filter's N + 1 row pointers are
+    checked before any launch.
+
+    The pairs are grouped by query node on the device; the distinct query nodes go through in blocks of
+    max(1, block_bytes // (8 N)) rows, one reused block buffer: their distance rows (ops.dist_rows; the bounded domain
+    on its inverse Cayley transform, once per table, as in evaluate), then the counts of every target of the block's
+    rows (ops.target_ranks).  Beyond the block it holds the kernels' workspaces and a few int64 / float64 arrays of E
+    entries.  world_size > 1: this rank takes its distributed.row_shard part of the distinct query nodes, so no
+    distance row is computed twice, and one SUM all-reduce of (sum of 1 / rank, hits per k, count) over the default
+    process group makes MRR, Hits@k and count global.  The status word is checked once, at the end.  Returns a
+    LinkPrediction."""
+    if not isinstance(table, torch.Tensor):
+        raise TypeError("table must be a tensor")
+    if not isinstance(pairs, torch.Tensor) or pairs.dtype != torch.int64:
+        raise TypeError("pairs must be an int64 tensor")
+    if pairs.dim() != 2 or pairs.shape[1] != 2:
+        raise ValueError("pairs must have shape (E, 2)")
+    n_nodes = table.shape[0]
+    if pairs.numel() and (int(pairs.min()) < 0 or int(pairs.max()) >= n_nodes):
+        raise ValueError(f"pairs must lie in [0, {n_nodes})")
+    if bool((pairs[:, 0] == pairs[:, 1]).any()):
+        raise ValueError("pairs must not hold u == v")
+    ks = tuple(int(k) for k in ks)
+    if any(k < 1 for k in ks):
+        raise ValueError("every k of ks must be >= 1")
+    f_ptr, f_idx = filter_adj
+    if torch.as_tensor(f_ptr).numel() != n_nodes + 1:
+        raise ValueError(f"filter_adj must hold the CSR adjacency of all {n_nodes} nodes (N + 1 row pointers)")
+    table = _cuda_table("link_prediction", table)
+    dev = table.device
+    with torch.cuda.device(dev):
+        filt = _adjacency_on(filter_adj, dev)
+        pairs = pairs.to(dev)
+        e_all = pairs.shape[0]
+        # group by query node: positions sorted by source (stable), the distinct sources with a target CSR
+        order = torch.sort(pairs[:, 0], stable=True).indices
+        nodes, counts = torch.unique_consecutive(pairs[order, 0], return_counts=True)
+        t_ptr = torch.zeros(nodes.numel() + 1, dtype=torch.int64, device=dev)
+        torch.cumsum(counts, 0, out=t_ptr[1:])
+        t_idx = pairs[order, 1].contiguous()
+        lo, hi = 0, nodes.numel()
+        if world_size > 1:
+            lo, hi, _ = sd.row_shard(nodes.numel(), rank, world_size)
+        e0, e1 = (int(x) for x in t_ptr[[lo, hi]].tolist())
+        lt = torch.full((e_all,), -1, dtype=torch.int64, device=dev)
+        le = torch.full((e_all,), -1, dtype=torch.int64, device=dev)
+        if hi > lo:
+            src, kind, metric, wsum = _distance_source(manifold, table)
+            block = max(1, min(block_bytes // (8 * n_nodes), hi - lo))
+            buf = torch.empty(block * n_nodes, dtype=torch.float64, device=dev)
+            for q0 in range(lo, hi, block):
+                qc = min(block, hi - q0)
+                q = nodes[q0:q0 + qc]
+                d = ops.dist_rows(kind, metric, src, q, wsum, out=buf[: qc * n_nodes].view(qc, n_nodes))
+                ops.target_ranks(d, q, (t_ptr[q0:q0 + qc + 1], t_idx), filt, out=(lt, le))
+            del buf, src
+        positions, back = torch.sort(order[e0:e1])
+        lt, le = lt[e0:e1][back].to(torch.float64), le[e0:e1][back].to(torch.float64)
+        undefined = lt < 0
+        optimistic = (1.0 + lt).masked_fill_(undefined, math.nan)
+        pessimistic = (1.0 + le).masked_fill_(undefined, math.nan)
+        ranks = 1.0 + 0.5 * (lt + le)
+        ranks.masked_fill_(undefined, math.nan)
+        sums = torch.stack([(1.0 / ranks).sum()] + [(ranks <= k).sum().to(torch.float64) for k in ks]
+                           + [torch.tensor(float(e1 - e0), dtype=torch.float64, device=dev)])
+        if world_size > 1:
+            import torch.distributed as dist
+            dist.all_reduce(sums)
+        ops.check_status(dev)
+        sums = sums.tolist()
+    count = int(sums[-1])
+    mean = (lambda x: x / count) if count else (lambda x: math.nan)
+    return LinkPrediction(mrr=mean(sums[0]), hits={k: mean(h) for k, h in zip(ks, sums[1:-1])}, count=count,
+                          pairs=positions, rank=ranks, optimistic=optimistic, pessimistic=pessimistic)
 
 
 def sample_order(num_nodes, num_rows, *, seed=0, epoch=0, device=None):

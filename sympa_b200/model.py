@@ -76,6 +76,13 @@ class Model(nn.Module):
         from .metrics import nearest
         return nearest(self.manifold, self.embeddings.embeds, queries, k, scale=self._eval_scale(), **kw)
 
+    def link_prediction(self, pairs, filter_adj, **kw):
+        """Filtered link-prediction ranks of the directed query pairs `pairs` ((E, 2) int64) against the CSR adjacency
+        `filter_adj` of the known edges, with MRR and Hits@k: the metrics.LinkPrediction of
+        sympa_b200.metrics.link_prediction (see there for the keywords).  Ranks do not depend on the scale."""
+        from .metrics import link_prediction
+        return link_prediction(self.manifold, self.embeddings.embeds, pairs, filter_adj, **kw)
+
     def _eval_scale(self):
         with torch.no_grad():
             return float(self.get_scale().item())

@@ -674,6 +674,63 @@ def row_topk(dist_block, k, exclude=None, out=None):
     return out
 
 
+_rank_workspace = {}
+
+
+def target_ranks(dist_block, queries, targets, filter_adj, out=None):
+    """Filtered ranks of held-out targets among all N nodes: sympa_target_ranks.  dist_block: the (R, N) float64 block
+    of the distance rows of `queries` ((R,) int64; what dist_rows returns).  targets = (ptr, idx): int64, ptr with
+    R + 1 entries, the targets of block row r are idx[ptr[r]:ptr[r + 1]].  filter_adj = (ptr, idx): the CSR adjacency
+    of all N nodes whose row u lists the known neighbours of u (graphs.adjacency_csr), left out of the competitors.
+    All on the block's device.  Returns (lt, le): int64 tensors shaped like targets' idx, entry i the number of
+    competitors strictly closer than, and at most as far as, the target idx[i] (definition in include/sympa_b200.h);
+    -1 for every pair of a row with a NaN distance (which sets the non-finite status bit).  Only the entries
+    [ptr[0], ptr[R]) are written; `out` = (lt, le) to write into, otherwise they are allocated filled with -1.  The
+    workspace (8 bytes per row and 24 per entry of idx) is kept per device and reused."""
+    lib = _lib.load()
+    dist_block = _require(dist_block, "dist_block")
+    if dist_block.dim() != 2:
+        raise ValueError("dist_block must be (rows, N)")
+    rows, n_cols = dist_block.shape
+    dev = dist_block.device
+    queries = _require(queries, "queries", torch.int64)
+    t_ptr, t_idx = (_require(t, name, torch.int64) for t, name in zip(targets, ("targets ptr", "targets idx")))
+    f_ptr, f_idx = (_require(t, name, torch.int64) for t, name in zip(filter_adj, ("filter ptr", "filter idx")))
+    if any(t.device != dev for t in (queries, t_ptr, t_idx, f_ptr, f_idx)):
+        raise ValueError("queries, targets and the filter must be on the distance block's device")
+    if tuple(queries.shape) != (rows,):
+        raise ValueError(f"queries must have shape ({rows},)")
+    if t_ptr.dim() != 1 or t_ptr.numel() != rows + 1 or t_idx.dim() != 1:
+        raise ValueError(f"targets ptr must have R + 1 = {rows + 1} entries and idx must be 1-D")
+    if f_ptr.dim() != 1 or f_ptr.numel() != n_cols + 1 or f_idx.dim() != 1:
+        raise ValueError(f"filter ptr must have N + 1 = {n_cols + 1} entries and idx must be 1-D")
+    if out is None:
+        out = (torch.full_like(t_idx, -1), torch.full_like(t_idx, -1))
+    else:
+        lt, le = out
+        if any(o.dtype != torch.int64 or o.device != dev or o.shape != t_idx.shape or not o.is_contiguous()
+               for o in (lt, le)):
+            raise ValueError(f"out must be two contiguous int64 ({t_idx.numel()},) tensors on {dev}")
+    if rows == 0 or n_cols == 0:
+        return out
+    with torch.cuda.device(dev):
+        nbytes = lib.sympa_target_ranks_workspace_bytes(rows, t_idx.numel())
+        key = (dev.type, dev.index if dev.index is not None else torch.cuda.current_device())
+        ws = _rank_workspace.get(key)
+        if ws is None or ws.numel() * 8 < nbytes:
+            ws = torch.empty(nbytes // 8, dtype=torch.float64, device=dev)
+            _rank_workspace[key] = ws
+        dummy = None
+        if t_idx.numel() == 0 or f_idx.numel() == 0:
+            dummy = torch.zeros(1, dtype=torch.int64, device=dev)      # no entries: any valid pointer
+        _lib.check(lib.sympa_target_ranks(rows, n_cols, _ptr(dist_block), _ptr(queries), _ptr(t_ptr),
+                                          _ptr(t_idx if t_idx.numel() else dummy), _ptr(f_ptr),
+                                          _ptr(f_idx if f_idx.numel() else dummy), _ptr(out[0] if out[0].numel() else dummy),
+                                          _ptr(out[1] if out[1].numel() else dummy), _ptr(ws), ws.numel() * 8,
+                                          _ptr(status_word(dev)), _stream()))
+    return out
+
+
 _ap_workspace = {}
 
 

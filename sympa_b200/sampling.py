@@ -53,11 +53,14 @@ def _mix_tensor(x):
     return x ^ _shr(x, 31)
 
 
-def source_keys(seed, epoch, nodes, tag=1):
-    """h(seed, epoch, tag, node, 0) of every node of the int64 tensor `nodes`, as int64 tensors whose signed order is
-    the unsigned order of the hash.  Tag 1 orders the training sources, tag 2 the nodes metrics.estimate samples."""
+def source_keys(seed, epoch, nodes, tag=1, second=None):
+    """h(seed, epoch, tag, node, 0) of every node of the int64 tensor `nodes`, or h(seed, epoch, tag, node, b) with b
+    the matching entry of the int64 tensor `second`, as int64 tensors whose signed order is the unsigned order of the
+    hash.  Tag 1 orders the training sources, tag 2 the nodes metrics.estimate samples, tag 3 (with the second
+    endpoint) the edges graphs.split_edges holds out."""
     head = _i64(_mix(_mix(_mix(seed) ^ epoch) ^ tag))
-    h = _mix_tensor(_mix_tensor(nodes ^ head))
+    h = _mix_tensor(nodes ^ head)
+    h = _mix_tensor(h if second is None else h ^ second)
     return h ^ _i64(1 << 63)
 
 
